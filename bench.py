@@ -19,6 +19,12 @@ the reference's torch code) timed on this box's host cores on a bounded sample.
 exist on the GPU box) on the host cores with all threads; rank 0 only.  It imports only torch, the oracle and the
 torch-only generator module gdsynth: libgdeconv.so is never mapped in that process.
 
+--dump-outputs DIR: after the timed steps, write what the last timed step of the headline path computed, as float32 .npy
+files: DIR/deconvolved.npy (rank 0's deconvolved stamps [S,1,48,48]) and DIR/ellipticities.npy (the gathered moment
+ellipticities [S,2]).  Arrays longer than 4096 stamps / 2^21 galaxies are cut to a fixed seeded sample of that many rows in
+index order (at most 55 MB in all).  Inputs and weights are seeded, so two builds run with the same arguments can be compared
+file for file.
+
 --config 3|4|5 run the other BASELINE.json configs (one JSON line per measurement; the default line, config 2, is unchanged):
   3  Unrolled-ADMM(8) on --total (1,000,000) stamps, STRONG scaling: the total is sharded by galaxy over the ranks, every shard
      is generated on its own GPU, and one step = forward over the whole shard + moment ellipticities + NCCL all-gather;
@@ -101,6 +107,14 @@ class ClockSampler:
         return dict(sm_mhz=sm[len(sm) // 2] if sm else None, sm_max_mhz=mx or None, reasons=sorted(reasons), samples=len(sm))
 
 
+def seeded_rows(t, k, seed=0):
+    """t itself if it has at most k rows, else k of its rows picked by a fixed seed, in index order."""
+    if t.shape[0] <= k:
+        return t
+    idx = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(seed))[:k].sort().values
+    return t[idx.to(t.device)]
+
+
 def cpu_reference(n_iters, sample, batch, steps, warmup):
     """The reference's CPU implementation of the path (oracle port, bit-exact vs the reference) on the host cores."""
     import oracle.ref_models as O
@@ -138,7 +152,12 @@ def main():
     ap.add_argument('--total', type=int, default=1000000, help='configs 3/4: total stamps over all ranks')
     ap.add_argument('--sweep-stamps', type=int, default=100000, help='config 5: stamps per sweep point over all ranks')
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs of the last timed step as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'b200' or args.config != 2):
+        ap.error('--dump-outputs covers the headline path only (--impl b200, --config 2)')
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
     local = int(os.environ.get('LOCAL_RANK', 0))
@@ -197,7 +216,7 @@ def main():
 
     def step_device():
         out = model(obs, psf, alpha)
-        return gather_ellipticities(moments_e(out), n_total)
+        return out, gather_ellipticities(moments_e(out), n_total)
 
     def step_e2e():
         # the public host-batch call: chunk-pipelined H2D / compute / D2H inside the engine (one cudaMemcpyAsync per tensor and
@@ -207,8 +226,11 @@ def main():
         e_host.copy_(e, non_blocking=True)
 
     def timed(fn, steps, warmup):
+        """-> (ms per step, launches in the timed steps, what the last timed step returned).  The warm-up keeps each step's
+        result alive through the next step exactly like the timed loop, so the allocator holds both before timing starts."""
+        last = None
         for _ in range(warmup):
-            fn()
+            last = fn()
         torch.cuda.synchronize()
         if world > 1:
             dist.barrier()
@@ -217,7 +239,7 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            last = fn()
         e1.record()
         torch.cuda.synchronize()
         if world > 1:
@@ -226,12 +248,16 @@ def main():
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms) / steps, int(lib.gd_launch_count() - l0)
+        return float(ms) / steps, int(lib.gd_launch_count() - l0), last
 
     with ClockSampler(local) as clk:
-        ms_step, launches = timed(step_device, args.steps, max(3, args.warmup))
+        ms_step, launches, (out_last, e_last) = timed(step_device, args.steps, max(3, args.warmup))
     clocks = clk.summary()
-    ms_e2e, _ = timed(step_e2e, args.steps, max(3, args.warmup))
+    dump = None
+    if args.dump_outputs and rank == 0:
+        dump = dict(deconvolved=seeded_rows(out_last, 4096).float().cpu(), ellipticities=seeded_rows(e_last, 1 << 21).float().cpu())
+    del out_last, e_last
+    ms_e2e, _, _ = timed(step_e2e, args.steps, max(3, args.warmup))
 
     # dominant kernel, live: every k_conv_umma / k_rb_umma launch of one more step bracketed by CUDA events on its stream
     roof = None
@@ -290,6 +316,11 @@ def main():
     if world == 1 and not args.no_cpu_baseline:
         r = cpu_reference(args.n_iters, args.cpu_sample, 64, 3, 1)
         line['cpu_baseline'] = {k: r[k] for k in ('value', 'unit', 'cores', 'kind', 'sample')}
+    if dump:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + '.npy'), t.numpy())
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -17,7 +17,7 @@ import oracle.ref_models as O
 from conftest import ROOT, rel_l2
 
 PKG = os.path.join(ROOT, 'galaxy-deconv_b200')
-REF = '/root/reference'
+REF = os.environ.get('GDECONV_REFERENCE', '')       # a checkout of the upstream Galaxy-Deconv project, if one is at hand
 
 
 def test_models_and_utils_are_namespace_packages():
@@ -72,10 +72,10 @@ print('DROPIN-OK')
 '''
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'models')), reason='reference checkout not mounted (GPU box)')
-def test_reference_drivers_import_unchanged_on_top_of_this_package():
+@pytest.mark.skipif(not REF or not os.path.isdir(os.path.join(REF, 'models')), reason='GDECONV_REFERENCE names no upstream checkout')
+def test_reference_drivers_import_unchanged_on_top_of_this_package(tmp_path):
     env = {k: v for k, v in os.environ.items() if k != 'PYTHONPATH'}
-    r = subprocess.run([sys.executable, '-c', CHILD, PKG, REF], capture_output=True, text=True, timeout=300, env=env, cwd='/tmp')
+    r = subprocess.run([sys.executable, '-c', CHILD, PKG, REF], capture_output=True, text=True, timeout=300, env=env, cwd=tmp_path)
     assert r.returncode == 0 and 'DROPIN-OK' in r.stdout, r.stderr[-3000:]
 
 

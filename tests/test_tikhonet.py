@@ -11,6 +11,8 @@ import torch
 import oracle.ref_models as O
 from conftest import ROOT, rel_l2
 
+REF = os.environ.get('GDECONV_REFERENCE', '')       # a checkout of the upstream Galaxy-Deconv project, if one is at hand
+
 
 @pytest.fixture(scope='module')
 def tik():
@@ -45,7 +47,7 @@ def test_state_dict_layout_matches_reference_file(tik):
     assert list(a.keys()) == list(b.keys()) and all(torch.equal(a[k], b[k]) for k in a)
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/saved_models'), reason='reference checkout not mounted')
+@pytest.mark.skipif(not REF or not os.path.isdir(os.path.join(REF, 'saved_models')), reason='GDECONV_REFERENCE names no upstream checkout')
 def test_golden_regenerates_from_live_reference():
     r = subprocess.run([sys.executable, os.path.join(ROOT, 'tests', 'golden', 'make_golden_tikhonet.py'), '--check'],
                        capture_output=True, text=True, timeout=600)
