@@ -196,6 +196,7 @@ static int init_once(int device) {
     GD_TRY(conv_rb_init());
     GD_TRY(conv_l1chain_init());
     GD_TRY(conv_l2chain_init());
+    GD_TRY(synth_init());
     done.fetch_or(1u << device);
     return GD_OK;
 }
@@ -898,6 +899,24 @@ extern "C" int gd_conv_otf(const float* otf, int otf_batch, const float* x, floa
 extern "C" int gd_moments_e(const float* img, float* e12, int batch, void* stream) {
     if (batch < 0 || (batch && (!img || !e12))) GD_FAIL(GD_EBADSHAPE, "gd_moments_e: bad batch or NULL buffers");
     return launch_moments(img, e12, batch, (cudaStream_t)stream);
+}
+
+extern "C" int gd_synth_batch(int64_t start, int count, int64_t seed, int snr_mode, float snr, float psf_fwhm_err,
+                              float psf_shear_err, float* obs, float* psf, float* alpha, float* gt, void* stream) {
+    if (count < 0) GD_FAIL(GD_EBADSHAPE, "gd_synth_batch: count %d < 0", count);
+    if (!obs && !psf && !alpha && !gt) GD_FAIL(GD_EBADSHAPE, "gd_synth_batch: every output is NULL");
+    if (snr_mode != GD_SYNTH_SNR_FIXED && snr_mode != GD_SYNTH_SNR_MIXED)
+        GD_FAIL(GD_EBADSHAPE, "gd_synth_batch: unknown snr_mode %d", snr_mode);
+    if (snr_mode == GD_SYNTH_SNR_FIXED && !(snr > 0.f && isfinite(snr)))
+        GD_FAIL(GD_EBADSHAPE, "gd_synth_batch: snr must be positive and finite in fixed mode, got %g", (double)snr);
+    if (start < 0 || start > INT64_MAX - count) GD_FAIL(GD_EBADSHAPE, "gd_synth_batch: stamp range [%lld, +%d) out of range", (long long)start, count);
+    if (!isfinite(psf_fwhm_err) || !isfinite(psf_shear_err)) GD_FAIL(GD_EBADSHAPE, "gd_synth_batch: non-finite PSF error");
+    if (count == 0) return GD_OK;
+    int dev;
+    GD_CUDA_CHECK(cudaGetDevice(&dev));
+    GD_TRY(init_once(dev));
+    return launch_synth(start, count, seed, snr_mode == GD_SYNTH_SNR_MIXED, snr, psf_fwhm_err, psf_shear_err, obs, psf, alpha, gt,
+                        (cudaStream_t)stream);
 }
 
 extern "C" int gd_debug_geom(int H, int batch, int* geom7) {

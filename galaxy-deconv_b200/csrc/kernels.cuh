@@ -1,5 +1,5 @@
 // Host-callable launchers of every kernel in libgdeconv (definitions in fft_kernels.cu, subnet.cu, conv_simt.cu,
-// conv_umma.cu).  All are stream-ordered and return GD_OK or a negative GD_E* code.
+// conv_umma.cu, synth.cu).  All are stream-ordered and return GD_OK or a negative GD_E* code.
 #pragma once
 #include "gd_common.cuh"
 #include "subnet.cuh"
@@ -51,6 +51,9 @@ int launch_u_post(const float2* Hw, const float* rho, int n_rho, int n, int it, 
 int launch_scale_by_alpha(float* out, const float* x, const float* alpha, int batch, int use_alpha, cudaStream_t st);
 int launch_moments(const float* img, float* e12, int batch, cudaStream_t st);
 int launch_subnet(const SubnetParams& P, const float* psf, const float* alpha, float* rho, int batch, cudaStream_t st);
+int synth_init();
+int launch_synth(int64_t start, int count, int64_t seed, int mixed, float snr, float fwhm_err, float shear_err, float* obs,
+                 float* psf, float* alpha, float* gt, cudaStream_t st);
 
 int launch_conv_simt(const ConvParams& p, int prec, cudaStream_t st);
 int launch_conv_umma(const ConvParams& p, cudaStream_t st);

@@ -2,3 +2,4 @@
 from . import _lib  # noqa: F401  (loads / builds the shared library; fails loudly if it cannot)
 from .engine import (AdmmEngine, conv_fft_batch, fft_solver, moments_e, require_cuda_stamps, resunet_forward,  # noqa: F401
                      launch_count, default_precision)
+from .synth import make_batch_device  # noqa: F401

@@ -522,6 +522,13 @@ def moments_e(img):
     return e
 
 
+def synth_batch(device, start, count, seed, snr_mode, snr, psf_fwhm_err, psf_shear_err, obs=None, psf=None, alpha=None, gt=None):
+    """gd_synth_batch on `device`'s current stream into preallocated contiguous fp32 CUDA tensors (any may be None, not all)."""
+    with torch.cuda.device(device):
+        check(lib.gd_synth_batch(int(start), int(count), int(seed), int(snr_mode), float(snr), float(psf_fwhm_err), float(psf_shear_err),
+                                 _ptr(obs), _ptr(psf), _ptr(alpha), _ptr(gt), _stream(device)))
+
+
 # ---------------------------------------------------------------------------------------------------
 # XDenseUNet / Tikhonet (csrc/xdense.cu)
 # ---------------------------------------------------------------------------------------------------

@@ -148,6 +148,20 @@ GD_API int gd_admm_forward_xdense(const GdWeights* w, const GdXDense* x, int llh
                                   const float* alpha, float* out, float* rho_out, float* analysis, int batch, void* workspace,
                                   size_t workspace_bytes, void* xd_workspace, size_t xd_workspace_bytes, int xd_chunk, void* stream);
 
+/* Synthetic galaxy stamps on the device: the CUDA twin of the generator module gdsynth.py (make_batch), which stands in for the
+ * reference's GalSim pipeline (generate_data.py:114-334) and keeps its conventions: 48x48 stamps rendered 4x oversampled and
+ * averaged 4x4 (utils/utils_data.py:26-40), Sersic galaxy, Moffat PSF centred on pixel (24,24), sky + read noise sigma = 19.04
+ * ADU, flux scaled to the SNR, obs = max(gt (*) psf, 0) + N(0, sigma^2) and alpha = obs.mean() (utils/utils_data.py:100-101).
+ * Stamp i of the batch is stamp `start + i` of the stream `seed`: its values depend only on (seed, start + i).
+ *   snr_mode  GD_SYNTH_SNR_FIXED: every stamp at `snr` (> 0);  GD_SYNTH_SNR_MIXED: log-uniform in [20, 300] per stamp
+ *   psf_fwhm_err (arcsec) / psf_shear_err: when either is non-zero, `psf` is the mismatched model PSF while obs was blurred
+ *             with the true one (the PSF-mismatch sweep of test_psf.py:237,242)
+ *   obs, psf, gt [count][48*48] fp32 device, alpha [count] fp32 device; `psf` sums to 1/16.  Any output may be NULL (not all):
+ *             only the stages the requested outputs need run, so a psf-only call renders just the PSF. */
+enum { GD_SYNTH_SNR_FIXED = 0, GD_SYNTH_SNR_MIXED = 1 };
+GD_API int gd_synth_batch(int64_t start, int count, int64_t seed, int snr_mode, float snr, float psf_fwhm_err,
+                          float psf_shear_err, float* obs, float* psf, float* alpha, float* gt, void* stream);
+
 /* Test hook: one tap-GEMM layer of the denoiser on caller-packed operands (layouts of csrc/gd_common.cuh:
  * activations [Kt/CH][Ptot][CH], CH = 8 halves (fp16 modes) or 4 floats; weights as gd_pack_weights lays them out
  * for `precision`; out32 [N/4][Ptot][4] fp32).  ntaps = 9 (3x3, zero padding) or 1.  `geom7` receives
