@@ -919,6 +919,18 @@ extern "C" int gd_synth_batch(int64_t start, int count, int64_t seed, int snr_mo
                         (cudaStream_t)stream);
 }
 
+extern "C" int gd_adaptive_moments(const float* img, int batch, float guess_sigma, float* shape, int32_t* info, void* stream) {
+    if (batch < 0) GD_FAIL(GD_EBADSHAPE, "gd_adaptive_moments: batch %d < 0", batch);
+    if (batch && (!img || !shape || !info)) GD_FAIL(GD_EBADSHAPE, "gd_adaptive_moments: NULL buffer for a batch of %d", batch);
+    if (!(isfinite(guess_sigma) && guess_sigma > 0.f && guess_sigma <= 24.f))
+        GD_FAIL(GD_EBADSHAPE, "gd_adaptive_moments: guess_sigma must be finite and in (0, 24] px, got %g", (double)guess_sigma);
+    if (batch == 0) return GD_OK;
+    int dev;
+    GD_CUDA_CHECK(cudaGetDevice(&dev));
+    GD_TRY(init_once(dev));
+    return launch_adaptive_moments(img, batch, guess_sigma, shape, info, (cudaStream_t)stream);
+}
+
 extern "C" int gd_debug_geom(int H, int batch, int* geom7) {
     if (H < 1 || batch < 1 || !geom7) GD_FAIL(GD_EBADSHAPE, "gd_debug_geom: bad arguments");
     Geom g = make_geom(H, batch);

@@ -15,13 +15,15 @@ PREC_FP32_SIMT, PREC_FP16_UMMA, PREC_FP16_SIMT = 0, 1, 2
 LLH_GAUSSIAN, LLH_POISSON = 0, 1
 SOLVER_RL, SOLVER_WIENER, SOLVER_TIKHONOV_ID, SOLVER_TIKHONOV_LAP = 0, 1, 2, 3
 SYNTH_SNR_FIXED, SYNTH_SNR_MIXED = 0, 1
+SHAPE_OK, SHAPE_MAXITER, SHAPE_FLUX, SHAPE_MOMENTS, SHAPE_CENTROID = 0, 1, 2, 3, 4
 PRECISIONS = {'fp32_simt': PREC_FP32_SIMT, 'fp16_umma': PREC_FP16_UMMA, 'fp16_simt': PREC_FP16_SIMT}
 
 #: every symbol include/gdeconv.h declares (tests/test_abi.py checks the header against this list and the .so)
 SYMBOLS = ('gd_version', 'gd_last_error', 'gd_pack_weights', 'gd_free_weights', 'gd_workspace_bytes', 'gd_workspace_init', 'gd_workspace_release',
            'gd_admm_forward', 'gd_resunet_forward', 'gd_subnet_forward', 'gd_fft_solver', 'gd_conv_fft', 'gd_moments_e',
            'gd_launch_count', 'gd_debug_geom', 'gd_debug_tapgemm', 'gd_profile_begin', 'gd_profile_end', 'gd_pack_xdense', 'gd_free_xdense', 'gd_xdense_workspace_bytes',
-           'gd_xdense_forward', 'gd_tikhonet_forward', 'gd_admm_forward_xdense', 'gd_psf_to_otf', 'gd_conv_otf', 'gd_max_chunk', 'gd_debug_divmagic', 'gd_synth_batch')
+           'gd_xdense_forward', 'gd_tikhonet_forward', 'gd_admm_forward_xdense', 'gd_psf_to_otf', 'gd_conv_otf', 'gd_max_chunk', 'gd_debug_divmagic', 'gd_synth_batch',
+           'gd_adaptive_moments')
 
 
 class GdTensorDesc(C.Structure):
@@ -69,6 +71,7 @@ def _load():
     lib.gd_psf_to_otf.argtypes = [vp, i, i, i, vp, vp, i, vp]
     lib.gd_conv_otf.argtypes = [vp, i, vp, vp, i, vp]
     lib.gd_synth_batch.argtypes = [C.c_int64, i, C.c_int64, i, f, f, f, vp, vp, vp, vp, vp]
+    lib.gd_adaptive_moments.argtypes = [vp, i, f, vp, vp, vp]
     lib.gd_max_chunk.restype = i
     lib.gd_debug_divmagic.argtypes = [C.c_uint, C.c_uint, C.c_uint]
     lib.gd_debug_divmagic.restype = C.c_longlong

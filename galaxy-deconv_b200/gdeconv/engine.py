@@ -522,6 +522,24 @@ def moments_e(img):
     return e
 
 
+def adaptive_moments(img, guess_sigma=3.0):
+    """Adaptive second moments of every stamp (gd_adaptive_moments, csrc/shape.cu): an elliptical Gaussian weight, started at
+    pixel (24, 24) with sigma = ``guess_sigma`` px, iterated until it matches the stamp's own weighted centroid and second moments.
+    ``img`` is fp32 CUDA [B,1,48,48]; the work runs on the current stream of its device.  Returns a dict:
+    flux [B], centroid [B,2] (x, y; x = column), M [B,3] (Mxx, Mxy, Myy, px^2), e [B,2] (distortion, as moments_e),
+    sigma [B] = det(M)^(1/4), status [B] int32 (_lib.SHAPE_*: OK, MAXITER, FLUX, MOMENTS, CENTROID) and n_iter [B] int32 passes.
+    The floats are NaN wherever status is not OK."""
+    img = require_cuda_stamps('img', img)
+    B, dev = img.shape[0], img.device
+    shape = torch.empty(B, 8, device=dev)
+    info = torch.empty(B, 2, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        check(lib.gd_adaptive_moments(_ptr(img), B, float(guess_sigma), _ptr(shape), _ptr(info), _stream(dev)))
+        M = shape[:, 3:6]
+        sigma = (M[:, 0] * M[:, 2] - M[:, 1] * M[:, 1]).pow(0.25)
+    return dict(flux=shape[:, 0], centroid=shape[:, 1:3], M=M, e=shape[:, 6:8], sigma=sigma, status=info[:, 0], n_iter=info[:, 1])
+
+
 def synth_batch(device, start, count, seed, snr_mode, snr, psf_fwhm_err, psf_shear_err, obs=None, psf=None, alpha=None, gt=None):
     """gd_synth_batch on `device`'s current stream into preallocated contiguous fp32 CUDA tensors (any may be None, not all)."""
     with torch.cuda.device(device):

@@ -162,6 +162,21 @@ enum { GD_SYNTH_SNR_FIXED = 0, GD_SYNTH_SNR_MIXED = 1 };
 GD_API int gd_synth_batch(int64_t start, int count, int64_t seed, int snr_mode, float snr, float psf_fwhm_err,
                           float psf_shear_err, float* obs, float* psf, float* alpha, float* gt, void* stream);
 
+/* Adaptive second moments of each stamp (Bernstein & Jarvis 2002; Hirata & Seljak 2003; the estimator family of GalSim's
+ * galsim.hsm.FindAdaptiveMom, without its step damping and bounds).  Pixel p = 48 r + c is at x = c, y = r.  The weight
+ * w = exp(-rho^2/2), rho^2 = (Myy dx^2 - 2 Mxy dx dy + Mxx dy^2) / det(M) starts at (24, 24) with M = guess_sigma^2 I; each pass
+ * sets the centroid to the weighted centroid and M to twice the weighted central second moments, until the centroid moves by
+ * <= 1e-5 sqrt(t) and M by <= 1e-5 t (t = tr M / 2), at most 100 passes.  A stamp stops early with GD_SHAPE_FLUX when the
+ * weighted flux is not positive (or NaN), GD_SHAPE_MOMENTS when M is not positive definite or tr M > 1152 px^2, and
+ * GD_SHAPE_CENTROID when the centroid leaves the 15 px box around (24, 24).
+ *   img    [batch][48*48] fp32 device;  guess_sigma in (0, 24] px (3 is a good start for galaxies of 1.5-6 px)
+ *   shape  [batch][8] fp32 device: flux (= 2 x the weighted flux, exact for a Gaussian), x0, y0, Mxx, Mxy, Myy,
+ *          e1 = (Mxx - Myy)/(Mxx + Myy), e2 = 2 Mxy/(Mxx + Myy) (the distortion of gd_moments_e); all NaN unless GD_SHAPE_OK
+ *   info   [batch][2] int32 device: status (GD_SHAPE_*), number of passes made
+ * A stamp's result does not depend on the batch it is measured in. */
+enum { GD_SHAPE_OK = 0, GD_SHAPE_MAXITER = 1, GD_SHAPE_FLUX = 2, GD_SHAPE_MOMENTS = 3, GD_SHAPE_CENTROID = 4 };
+GD_API int gd_adaptive_moments(const float* img, int batch, float guess_sigma, float* shape, int32_t* info, void* stream);
+
 /* Test hook: one tap-GEMM layer of the denoiser on caller-packed operands (layouts of csrc/gd_common.cuh:
  * activations [Kt/CH][Ptot][CH], CH = 8 halves (fp16 modes) or 4 floats; weights as gd_pack_weights lays them out
  * for `precision`; out32 [N/4][Ptot][4] fp32).  ntaps = 9 (3x3, zero padding) or 1.  `geom7` receives
