@@ -1,9 +1,9 @@
 // C ABI of libgdeconv (include/gdeconv.h): weight packing, workspace layout, the ResUNet layer graph and the
 // unrolled-ADMM drivers.  Host code only; every kernel lives in fft_kernels.cu / subnet.cu / conv_*.cu.
+#include <array>
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <map>
 #include <mutex>
@@ -61,8 +61,6 @@ struct GdWeights {
     const void* body_rb[2][2];
     const void* up[3];                // k2s2 transposed conv C_{L+1} -> C_L (index = fine level L)
     const void* up_rb[3][2][2];
-    const void* up1_plain;            // C1 = 64: m_up2's transposed conv in the same plain order (conv_l2chain.cu)
-    const void* up0_plain;            // C0 = 32, tcgen05 path: m_up1's transposed conv with plain column order n = (dy*2+dx)*C0 + co (conv_l1chain.cu)
     gd::SubnetParams sub;
     const float* rho_param;           // [n_rho] when subnet=False
 };
@@ -143,29 +141,19 @@ static int pack_down(Blob& bl, const GdTensorDesc* t, int Ci, int Co, int prec, 
     return GD_OK;
 }
 // ConvTranspose2d k2 s2 [Ci][Co][2][2] -> one tap, N = (dy*2+dx)*Co + co    (resnet_basicblock.py:81-87)
-static int pack_up(Blob& bl, const GdTensorDesc* t, int Ci, int Co, int prec, size_t* off, const char* what) {
+// paired: columns ordered for the lane-paired stores of epi_up_unit (conv_epilogue.cuh), the order k_conv_umma's transposed
+// conv writes; the chain kernels (conv_l1chain.cu, conv_l2chain.cu) and the SIMT kernel read the plain order
+static int pack_up(Blob& bl, const GdTensorDesc* t, int Ci, int Co, int prec, bool paired, size_t* off, const char* what) {
     if (!shape_is(t, Ci, Co, 2, 2)) GD_FAIL(GD_EBADSHAPE, "weight %s: missing or not (%d,%d,2,2)", what, Ci, Co);
     std::vector<float> B((size_t)Ci * 4 * Co);
     for (int ci = 0; ci < Ci; ++ci)
         for (int co = 0; co < Co; ++co)
             for (int tp = 0; tp < 4; ++tp) {
-                // tcgen05 path: columns ordered for the lane-paired stores of epi_up_unit (conv_epilogue.cuh)
                 const int dy = tp >> 1, dx = tp & 1;
-                const int n = prec == PREC_FP16_UMMA ? dy * 2 * Co + (co / 16) * 32 + ((co % 16) / 4) * 8 + dx * 4 + (co % 4) : tp * Co + co;
+                const int n = paired ? dy * 2 * Co + (co / 16) * 32 + ((co % 16) / 4) * 8 + dx * 4 + (co % 4) : tp * Co + co;
                 B[(size_t)ci * 4 * Co + n] = t->data[((size_t)ci * Co + co) * 4 + tp];
             }
     *off = pack_tapgemm(bl, 1, Ci, 4 * Co, prec, B);
-    return GD_OK;
-}
-
-// the same transposed conv for the level-0 chain kernel: plain column order n = (dy*2+dx)*Co + co
-static int pack_up_plain(Blob& bl, const GdTensorDesc* t, int Ci, int Co, size_t* off, const char* what) {
-    if (!shape_is(t, Ci, Co, 2, 2)) GD_FAIL(GD_EBADSHAPE, "weight %s: missing or not (%d,%d,2,2)", what, Ci, Co);
-    std::vector<float> B((size_t)Ci * 4 * Co);
-    for (int ci = 0; ci < Ci; ++ci)
-        for (int co = 0; co < Co; ++co)
-            for (int tp = 0; tp < 4; ++tp) B[(size_t)ci * 4 * Co + tp * Co + co] = t->data[((size_t)ci * Co + co) * 4 + tp];
-    *off = pack_tapgemm(bl, 1, Ci, 4 * Co, PREC_FP16_UMMA, B);
     return GD_OK;
 }
 
@@ -193,7 +181,6 @@ static int init_once(int device) {
     GD_TRY(fft_kernels_init());
     GD_TRY(subnet_init());
     GD_TRY(conv_umma_init());
-    GD_TRY(conv_rb_init());
     GD_TRY(conv_l1chain_init());
     GD_TRY(conv_l2chain_init());
     GD_TRY(synth_init());
@@ -263,10 +250,10 @@ extern "C" int gd_pack_weights(int arch, int n_iters, const GdTensorDesc* tensor
             GD_TRY(pack_down(bl, F.net(key), C, 2 * C, precision, &off, key));
             slot(&W.down[L], off);
             snprintf(key, sizeof key, "m_up%d.0.weight", L + 1);
-            GD_TRY(pack_up(bl, F.net(key), 2 * C, C, precision, &off, key));
+            // tcgen05 path: on path G (C0 = 32) m_up1 and m_up2 run inside the chain kernels
+            const bool paired = precision == PREC_FP16_UMMA && !(C0 == 32 && L < 2);
+            GD_TRY(pack_up(bl, F.net(key), 2 * C, C, precision, paired, &off, key));
             slot(&W.up[L], off);
-            if (L == 0 && C == 32 && precision == PREC_FP16_UMMA) { GD_TRY(pack_up_plain(bl, F.net(key), 2 * C, C, &off, key)); slot(&W.up0_plain, off); }
-            if (L == 1 && C == 64 && precision == PREC_FP16_UMMA) { GD_TRY(pack_up_plain(bl, F.net(key), 2 * C, C, &off, key)); slot(&W.up1_plain, off); }
         }
         for (int blk = 0; blk < 2; ++blk)
             for (int j = 0; j < 2; ++j) {
@@ -412,7 +399,9 @@ static Ws ws_layout(unsigned char* base, int arch, int prec, int chunk) {
     }
     w.lc_scratch = C0 == 32 ? take(l1chain_scratch_bytes() > l2chain_scratch_bytes() ? l1chain_scratch_bytes() : l2chain_scratch_bytes()) : nullptr;
     w.tpad = (float*)take((size_t)w.g[0].Ptot * 4);
-    w.tail_part = (float*)take((size_t)(C0 / 16) * 9 * w.g[0].Ptot * 4);   // 32-channel units (conv_umma.cu) or 16-channel halves (conv_rb.cu)
+    // per-tap m_tail partial sums: k_conv_umma writes C0 / 32 units of 9 planes, k_l1_chain one unit.  The C0 / 16 units allocated
+    // are twice that; shrinking them would change what gd_workspace_bytes reports.
+    w.tail_part = (float*)take((size_t)(C0 / 16) * 9 * w.g[0].Ptot * 4);
     w.total = off;
     return w;
 }
@@ -462,221 +451,110 @@ static int run_conv(const ConvParams& p, int prec, cudaStream_t st) {
     return prec == PREC_FP16_UMMA ? launch_conv_umma(p, st) : launch_conv_simt(p, prec, st);
 }
 
-// Head/tail fusion of the tcgen05 path (GDECONV_FUSE_HT=0 restores the stored fp32 head output and the k_tail kernel).
-static int g_fuse_ht = -1;
-static int fuse_ht_mode() {
-    if (g_fuse_ht < 0) {
-        const char* e = getenv("GDECONV_FUSE_HT");
-        g_fuse_ht = e ? atoi(e) : 1;
-    }
-    return g_fuse_ht;
-}
-// Fused ResBlock kernel at the 32-channel level (conv_rb.cu); GDECONV_FUSE_RB=0 restores one launch per conv.
-static int g_fuse_rb = -1;
-static int fuse_rb_mode() {
-    if (g_fuse_rb < 0) {
-        const char* e = getenv("GDECONV_FUSE_RB");
-        g_fuse_rb = e ? atoi(e) : 1;
-    }
-    return g_fuse_rb;
-}
-// fp16 hi/lo residual stream on the tcgen05 path (ConvParams::res_hi); GDECONV_HILO=0 restores the fp32 stream buffers.
-static int g_hilo = -1;
-static int hilo_mode() {
-    if (g_hilo < 0) {
-        const char* e = getenv("GDECONV_HILO");
-        g_hilo = e ? atoi(e) : 1;
-    }
-    return g_hilo;
-}
-// m_tail(x1) as an 81-coefficient stencil of the denoiser input in k_tail_gather (GDECONV_TAILG=0: recompute x1 in the conv epilogue)
-static int g_tailg = -1;
-static int tail_g_mode() {
-    if (g_tailg < 0) {
-        const char* e = getenv("GDECONV_TAILG");
-        g_tailg = e ? atoi(e) : 1;
-    }
-    return g_tailg;
-}
-// m_head fused into k_g_xupdate (path G, tcgen05, C0 = 32, head/tail fusion); GDECONV_XHEAD=0: separate k_head32 launch
-static int g_xhead = -1;
-static int xhead_mode() {
-    if (g_xhead < 0) {
-        const char* e = getenv("GDECONV_XHEAD");
-        g_xhead = e ? atoi(e) : 1;
-    }
-    return g_xhead;
-}
-// Level-0 chain kernels (conv_l1chain.cu): m_head + the two ResBlocks of m_down1, and the two ResBlocks of m_up1 + the m_tail partial
-// sums, each as ONE launch with the intermediates in shared / tensor memory.  GDECONV_L1CHAIN=0 restores one launch per layer pair.
-static int g_l1chain = -1;
-static int l1chain_mode() {
-    if (g_l1chain < 0) {
-        const char* e = getenv("GDECONV_L1CHAIN");
-        g_l1chain = e ? atoi(e) : 1;
-    }
-    return g_l1chain;
-}
-static int g_fuse_ht_fwd();
-static bool l1chain_applies(const GdWeights* W) {
-    return l1chain_mode() && W->precision == PREC_FP16_UMMA && W->nc[0] == 32 && g_fuse_ht_fwd() && hilo_mode() && tail_g_mode();
-}
-// Level-1 chain kernel (conv_l2chain.cu): the two ResBlocks of m_down2 resp. m_up2 as one launch each.  GDECONV_L2CHAIN=0 restores the
-// per-conv launches at that level.
-static int g_l2chain = -1;
-static int l2chain_mode() {
-    if (g_l2chain < 0) {
-        const char* e = getenv("GDECONV_L2CHAIN");
-        g_l2chain = e ? atoi(e) : 1;
-    }
-    return g_l2chain;
-}
-static bool l2chain_applies(const GdWeights* W) {
-    return l2chain_mode() && l1chain_applies(W) && W->nc[1] == 64 && W->up1_plain;
-}
-static bool xhead_applies(const GdWeights* W) {
-    return xhead_mode() && W->precision == PREC_FP16_UMMA && W->nc[0] == 32 && g_fuse_ht_fwd() && !l1chain_applies(W);
-}
-
-static int resunet_chunk(const GdWeights* W, const Ws& ws, const float* t, const float* tscale, float* zout, int nb,
-                         cudaStream_t st, bool head_done = false) {
+// Two graphs, chosen by the precision mode:
+//   * fp16_umma, the tcgen05 graph.  The fp32 output x1 of m_head is never stored: the conv epilogues that consume it recompute it
+//     from the padded-linear input copy tpad (ConvParams::head_t), and m_tail runs as per-tap partial sums (ConvParams::tail_part)
+//     that k_tail_gather shifts and adds, with m_tail(x1) as an 81-coefficient stencil of t.  The residual stream travels as fp16
+//     hi/lo: the fp32 stream buffers p32a / p32b are replaced by hi = the fp16 operand copy a16 and lo = lo16.  On path G
+//     (C0 = 32) levels 0 and 1 run in the chain kernels (conv_l1chain.cu, conv_l2chain.cu), one launch per stage.
+//   * fp32_simt / fp16_simt, the validation graph: one launch per layer, fp32 stream buffers, k_head and k_tail.
+static int resunet_chunk(const GdWeights* W, const Ws& ws, const float* t, const float* tscale, float* zout, int nb, cudaStream_t st) {
     const int prec = W->precision;
     const Geom* g = ws.g;
     const int* C = ws.C;
-    // every activation buffer has 16-byte rows, so stamps [s0, ...) of level L start s0 * S_L * 16 bytes into each plane
-    auto at = [&](const void* base, int L, int s0) -> unsigned char* {
-        return base ? (unsigned char*)base + (size_t)s0 * g[L].S * 16 : nullptr;
-    };
-    // tcgen05 path: x1 is never stored in fp32; its consumers recompute it from tpad (ConvParams::head_t)
-    const bool fuse = prec == PREC_FP16_UMMA && fuse_ht_mode() && C[0] <= 64;
-    const bool hilo = prec == PREC_FP16_UMMA && hilo_mode();
-    const bool l1chain = l1chain_applies(W);      // level 0 runs in the two chain kernels: no separate head launch, no level-0 fp32 buffers
-    const bool l2chain = l2chain_applies(W);      // the ResBlock pairs of level 1 run in one chain launch each
-    if (!l1chain) {   // head (ResUNet.py:31): x1 = conv(t)  -> skip32[0] (fp32) + a16[0]
-        ConvParams p = conv_base(g[0], nb);
-        p.N = C[0]; p.out32 = fuse ? nullptr : ws.skip32[0]; p.out16 = ws.a16[0];
-        if (!(head_done && fuse))
-            GD_TRY(launch_head(t, W->head, C[0] <= 64 ? W->head_h : nullptr, C[0], p, nb, prec, fuse ? ws.tpad : nullptr, st));
-    }
-    auto at4 = [&](float* base, int s0) -> float* { return base + (size_t)s0 * g[0].S; };    // 4-byte rows of level 0
-    // one ResBlock (resnet_basicblock.py:69-71) on stamps [s0, s0+n): stream + conv(relu(conv(stream))) -> two layers
-    // fp16 input of the next resblock() call; nullptr = ws.a16[L].  The fused ResBlock kernel (conv_rb.cu) must not write its
-    // fp16 output over its own input (neighbouring work items still read it as halo), so pairs ping-pong a16 <-> t16.
-    const void* rb_in16 = nullptr;
-    auto rb_params = [&](int L, int s0, int n, const void* const* w2, const float* res, const float* skip, float* out32,
-                         void* out16, void* s2d, ConvParams* out) {
-        const void* in16 = rb_in16 ? rb_in16 : ws.a16[L];
-        void* mid16 = in16 == ws.t16[L] ? ws.a16[L] : ws.t16[L];          // intermediate ReLU(conv1(x)) (unfused launches only)
-        out[0] = conv3(g[L], n, C[L], at(in16, L, s0), w2[0], 1);
-        out[0].out16 = at(mid16, L, s0);
-        out[1] = conv3(g[L], n, C[L], at(mid16, L, s0), w2[1], 0);
-        out[1].res32 = (const float*)at(res, L, s0); out[1].skip32 = (const float*)at(skip, L, s0);
-        out[1].out32 = (float*)at(out32, L, s0); out[1].out16 = at(out16, L, s0);
-        if (s2d) { out[1].s2d = at(s2d, L + 1, s0); out[1].gc = g[L + 1]; out[1].gc.M = n * g[L + 1].S; }
-    };
-    // head/tail fusion hooks for the second conv of the next resblock() call (level 0, consumed once)
-    bool ht_res_is_head = false, ht_skip_is_head = false, ht_tail = false, ht_drop_skip = false;
-    auto resblock = [&](int L, int s0, int n, const void* const* w2, const float* res, const float* skip, float* out32,
-                        void* out16, void* s2d) -> int {
-        ConvParams p[2];
-        rb_params(L, s0, n, w2, res, skip, out32, out16, s2d, p);
-        if (ht_res_is_head || ht_skip_is_head) {
-            p[1].head_t = at4(ws.tpad, s0); p[1].head_w = W->head_h;
-            if (ht_res_is_head) p[1].res32 = nullptr; else p[1].skip32 = nullptr;
+    const bool fused = prec == PREC_FP16_UMMA;
+    const bool chain = fused && C[0] == 32;
+    // one ResBlock (resnet_basicblock.py:69-71) on ws.a16[L]: conv + ReLU -> ws.t16[L], conv + res (+ skip) -> out32 / out16 / s2d
+    auto resblock_params = [&](int L, const void* const* w2, const float* res, const float* skip, float* out32, void* out16, void* s2d,
+                               ConvParams* p) {
+        p[0] = conv3(g[L], nb, C[L], ws.a16[L], w2[0], 1);
+        p[0].out16 = ws.t16[L];
+        p[1] = conv3(g[L], nb, C[L], ws.t16[L], w2[1], 0);
+        p[1].res32 = res; p[1].skip32 = skip; p[1].out32 = out32; p[1].out16 = out16;
+        if (s2d) { p[1].s2d = s2d; p[1].gc = g[L + 1]; p[1].gc.M = nb * g[L + 1].S; }
+        if (fused) {
+            auto is_stream = [&](const float* q) { return q && (q == ws.p32a[L] || q == ws.p32b[L]); };
+            if (is_stream(p[1].res32)) { p[1].res_hi = p[0].a; p[1].res_lo = ws.lo16[L]; p[1].res32 = nullptr; }
+            if (is_stream(p[1].out32) && p[1].out16) { p[1].out_lo = ws.lo16[L]; p[1].out32 = nullptr; }
         }
-        if (ht_drop_skip) p[1].skip32 = nullptr;          // the U-Net skip x1 enters through the composite stencil of k_tail_gather
-        if (ht_tail) { p[1].tail_part = at4(ws.tail_part, s0); p[1].tail_w = W->tail_h; p[1].out32 = nullptr; p[1].out16 = nullptr; }
-        ht_res_is_head = ht_skip_is_head = ht_tail = ht_drop_skip = false;
-        rb_in16 = nullptr;
-        if (hilo) {           // stream values travel as fp16 hi (= the ResBlock's fp16 input / output) + fp16 lo
-            auto is_stream = [&](const float* q) {
-                return q && (q == (const float*)at(ws.p32a[L], L, s0) || (L < 3 && q == (const float*)at(ws.p32b[L], L, s0)));
-            };
-            if (is_stream(p[1].res32)) { p[1].res_hi = p[0].a; p[1].res_lo = at(ws.lo16[L], L, s0); p[1].res32 = nullptr; }
-            if (is_stream(p[1].out32) && p[1].out16) { p[1].out_lo = at(ws.lo16[L], L, s0); p[1].out32 = nullptr; }
-        }
-        // fused kernel, except (mode 1) for the two ResBlocks whose epilogue recomputes m_head / reduces against m_tail: those
-        // FMA-heavy epilogues are faster on the eight 32-channel epilogue warps of conv_umma.cu (profiles/README);
-        // GDECONV_FUSE_RB=2 fuses them too
-        if (prec == PREC_FP16_UMMA && fuse_rb_mode() && conv_rb_supported(p[0], p[1]) &&
-            (fuse_rb_mode() >= 2 || (!p[1].tail_part && !p[1].head_t)))
-            return launch_conv_rb(p[0], p[1], st);
-        if (p[0].a == p[0].out16 || p[1].a == p[1].out16) GD_FAIL(GD_EUNSUPPORTED, "resblock: in-place fp16 buffers need the fused kernel");
+    };
+    auto run_pair = [&](const ConvParams* p) -> int {
         GD_TRY(run_conv(p[0], prec, st));
         return run_conv(p[1], prec, st);
     };
-    // two consecutive ResBlocks of one level: one chained launch when all four layers' weights fit in shared memory
-    auto resblock_pair = [&](int L, int s0, int n, const void* const* wa, const void* const* wb, const float* res_a, float* out32_a,
-                             void* out16_a, const float* res_b, const float* skip_b, float* out32_b, void* out16_b, void* s2d_b) -> int {
-        const bool last_l0 = fuse && L == 0 && skip_b != nullptr;       // second ResBlock of m_up1: + x1, then m_tail
-        const bool first_ht = fuse && L == 0 && res_a == ws.skip32[0];        // first ResBlock of m_down1: residual = x1
-        if (first_ht) ht_res_is_head = true;
-        // the first ResBlock writes its fp16 output to t16 when it runs in the fused kernel (no in-place halo race)
-        const bool pingpong = prec == PREC_FP16_UMMA && fuse_rb_mode() && C[L] == 32 && out16_a == ws.a16[L] &&
-                              (fuse_rb_mode() >= 2 || !first_ht);
-        GD_TRY(resblock(L, s0, n, wa, res_a, nullptr, out32_a, pingpong ? ws.t16[L] : out16_a, nullptr));
-        if (last_l0) { ht_skip_is_head = !tail_g_mode(); ht_tail = true; ht_drop_skip = tail_g_mode() != 0; }
-        if (pingpong) rb_in16 = ws.t16[L];
-        return resblock(L, s0, n, wb, res_b, skip_b, out32_b, out16_b, s2d_b);
+    auto resblock = [&](int L, const void* const* w2, const float* res, const float* skip, float* out32, void* out16, void* s2d) -> int {
+        ConvParams p[2];
+        resblock_params(L, w2, res, skip, out32, out16, s2d, p);
+        return run_pair(p);
     };
-    auto down_stage = [&](int L, int s0, int n) -> int {          // m_down{L+1} (ResUNet.py:32-34)
-        if (L == 0 && l1chain) {
-            const void* w4[4] = {W->down_rb[0][0][0], W->down_rb[0][0][1], W->down_rb[0][1][0], W->down_rb[0][1][1]};
-            // ... and the k2s2 strided conv of m_down1 (its space-to-depth operand never leaves shared memory)
-            return launch_l1chain_down(g[0], g[1], n, t + (size_t)s0 * NPIX, W->head_h, w4, W->down[0], (float*)at(ws.skip32[1], 1, s0),
-                                       at(ws.a16[1], 1, s0), l2chain ? at(ws.lo16[1], 1, s0) : nullptr, st);
+    auto w4 = [](const void* const (*rb)[2]) -> std::array<const void*, 4> { return {rb[0][0], rb[0][1], rb[1][0], rb[1][1]}; };
+
+    // m_head (ResUNet.py:31): x1 = conv(t) -> skip32[0] (fp32, validation graph) + a16[0]; tpad (tcgen05 graph)
+    if (!chain) {
+        ConvParams p = conv_base(g[0], nb);
+        p.N = C[0]; p.out32 = fused ? nullptr : ws.skip32[0]; p.out16 = ws.a16[0];
+        GD_TRY(launch_head(t, W->head, C[0], p, nb, prec, fused ? ws.tpad : nullptr, st));
+    }
+    // m_down1..3 (ResUNet.py:32-34): two ResBlocks, then the k2s2 strided conv as a 1-tap GEMM on the space-to-depth copy
+    for (int L = 0; L < 3; ++L) {
+        if (chain && L == 0) {          // m_head + both ResBlocks + the strided conv (its operand never leaves shared memory)
+            GD_TRY(launch_l1chain_down(g[0], g[1], nb, t, W->head_h, w4(W->down_rb[0]).data(), W->down[0], ws.skip32[1], ws.a16[1],
+                                       ws.lo16[1], st));
+            continue;
         }
-        if (L == 1 && l2chain) {
-            const void* w4[4] = {W->down_rb[1][0][0], W->down_rb[1][0][1], W->down_rb[1][1][0], W->down_rb[1][1][1]};
-            // ... and the k2s2 strided conv of m_down2 (its space-to-depth operand never leaves shared memory)
-            return launch_l2chain(0, g[1], g[2], n, at(ws.a16[1], 1, s0), at(ws.lo16[1], 1, s0), w4, W->down[1], (float*)at(ws.skip32[2], 2, s0),
-                                  at(ws.a16[2], 2, s0), nullptr, nullptr, nullptr, nullptr, nullptr, st);
-        } else
-            GD_TRY(resblock_pair(L, s0, n, W->down_rb[L][0], W->down_rb[L][1], ws.skip32[L], ws.p32a[L], ws.a16[L], ws.p32a[L], nullptr,
-                                 nullptr, nullptr, ws.d16[L + 1]));
-        ConvParams p = conv_base(g[L + 1], n);         // k2s2 strided conv as a 1-tap GEMM on the space-to-depth copy
-        p.ntaps = 1; p.off[0] = 0; p.Kt = 4 * C[L]; p.N = C[L + 1]; p.a = at(ws.d16[L + 1], L + 1, s0); p.w = W->down[L];
-        p.out32 = (float*)at(ws.skip32[L + 1], L + 1, s0); p.out16 = at(ws.a16[L + 1], L + 1, s0);
-        return run_conv(p, prec, st);
-    };
-    auto up_stage = [&](int L, int s0, int n) -> int {            // m_up{L+1} (ResUNet.py:36-38)
-        if (L == 0 && l1chain) {          // transposed conv + both ResBlocks + m_tail partial sums in one launch
-            const void* w4[4] = {W->up_rb[0][0][0], W->up_rb[0][0][1], W->up_rb[0][1][0], W->up_rb[0][1][1]};
-            return launch_l1chain_up(g[0], g[1], n, at(ws.a16[1], 1, s0), W->up0_plain, W->tail_h, w4, at4(ws.tail_part, s0), ws.lc_scratch, st);
+        if (chain && L == 1) {          // both ResBlocks + the strided conv
+            GD_TRY(launch_l2chain(0, g[1], g[2], nb, ws.a16[1], ws.lo16[1], w4(W->down_rb[1]).data(), W->down[1], ws.skip32[2], ws.a16[2],
+                                  nullptr, nullptr, nullptr, nullptr, nullptr, st));
+            continue;
         }
-        if (L == 1 && l2chain) {          // transposed conv + both ResBlocks + U-Net skip in one launch
-            const void* w4[4] = {W->up_rb[1][0][0], W->up_rb[1][0][1], W->up_rb[1][1][0], W->up_rb[1][1][1]};
-            return launch_l2chain(1, g[1], g[2], n, nullptr, nullptr, w4, nullptr, nullptr, nullptr, at(ws.a16[2], 2, s0), W->up1_plain, ws.lc_scratch,
-                                  (const float*)at(ws.skip32[1], 1, s0), at(ws.a16[1], 1, s0), st);
-        }
-        ConvParams p = conv_base(g[L + 1], n);         // k2s2 transposed conv: GEMM on the coarse level, scatter to fine
-        p.ntaps = 1; p.off[0] = 0; p.Kt = C[L + 1]; p.N = 4 * C[L]; p.a = at(ws.a16[L + 1], L + 1, s0); p.w = W->up[L];
-        p.mode = 1; p.Cf = C[L]; p.Cf_log2 = 0; while ((1 << p.Cf_log2) < p.Cf) ++p.Cf_log2; p.gf = g[L]; p.gf.M = n * g[L].S;
-        p.out32 = (float*)at(ws.p32a[L], L, s0); p.out16 = at(ws.a16[L], L, s0);
-        if (hilo) { p.out_lo = at(ws.lo16[L], L, s0); p.out32 = nullptr; }
-        GD_TRY(run_conv(p, prec, st));
-        if (L > 0) return resblock_pair(L, s0, n, W->up_rb[L][0], W->up_rb[L][1], ws.p32a[L], ws.p32b[L], ws.a16[L], ws.p32b[L],
-                                        ws.skip32[L], nullptr, ws.a16[L], nullptr);
-        return resblock_pair(L, s0, n, W->up_rb[L][0], W->up_rb[L][1], ws.p32a[L], ws.p32b[L], ws.a16[L], ws.p32b[L], ws.skip32[L],
-                             ws.p32a[L], nullptr, nullptr);
-    };
-    GD_TRY(down_stage(0, 0, nb));
-    GD_TRY(down_stage(1, 0, nb));
-    GD_TRY(down_stage(2, 0, nb));
+        ConvParams p[2];
+        resblock_params(L, W->down_rb[L][0], ws.skip32[L], nullptr, ws.p32a[L], ws.a16[L], nullptr, p);
+        if (fused && L == 0) { p[1].res32 = nullptr; p[1].head_t = ws.tpad; p[1].head_w = W->head_h; }     // residual x1, recomputed
+        GD_TRY(run_pair(p));
+        GD_TRY(resblock(L, W->down_rb[L][1], ws.p32a[L], nullptr, nullptr, nullptr, ws.d16[L + 1]));
+        ConvParams d = conv_base(g[L + 1], nb);
+        d.ntaps = 1; d.off[0] = 0; d.Kt = 4 * C[L]; d.N = C[L + 1]; d.a = ws.d16[L + 1]; d.w = W->down[L];
+        d.out32 = ws.skip32[L + 1]; d.out16 = ws.a16[L + 1];
+        GD_TRY(run_conv(d, prec, st));
+    }
     // m_body (ResUNet.py:35) and the skip x + x4 (:36)
-    GD_TRY(resblock(3, 0, nb, W->body_rb[0], ws.skip32[3], nullptr, ws.p32a[3], ws.a16[3], nullptr));
-    GD_TRY(resblock(3, 0, nb, W->body_rb[1], ws.p32a[3], ws.skip32[3], nullptr, ws.a16[3], nullptr));
-    GD_TRY(up_stage(2, 0, nb));
-    GD_TRY(up_stage(1, 0, nb));
-    GD_TRY(up_stage(0, 0, nb));
-    // tail (ResUNet.py:39): conv(x + x1), times the per-stamp input scale
-    if (l1chain) return launch_tail_gather(ws.tail_part, 1, g[0], tscale, zout, nb, t, W->tail_head_g, st, 1);
-    if (fuse) return launch_tail_gather(ws.tail_part, (fuse_rb_mode() >= 2 && C[0] == 32) ? 2 : C[0] / 32, g[0], tscale, zout, nb,
-                                        ws.tpad, tail_g_mode() ? W->tail_head_g : nullptr, st);
+    GD_TRY(resblock(3, W->body_rb[0], ws.skip32[3], nullptr, ws.p32a[3], ws.a16[3], nullptr));
+    GD_TRY(resblock(3, W->body_rb[1], ws.p32a[3], ws.skip32[3], nullptr, ws.a16[3], nullptr));
+    // m_up3..1 (ResUNet.py:36-38): the k2s2 transposed conv (GEMM on the coarse level, scattered to the fine one), two ResBlocks,
+    // the U-Net skip
+    for (int L = 2; L >= 0; --L) {
+        if (chain && L == 1) {          // transposed conv + both ResBlocks + U-Net skip
+            GD_TRY(launch_l2chain(1, g[1], g[2], nb, nullptr, nullptr, w4(W->up_rb[1]).data(), nullptr, nullptr, nullptr, ws.a16[2], W->up[1],
+                                  ws.lc_scratch, ws.skip32[1], ws.a16[1], st));
+            continue;
+        }
+        if (chain && L == 0) {          // transposed conv + both ResBlocks + the m_tail partial sums
+            GD_TRY(launch_l1chain_up(g[0], g[1], nb, ws.a16[1], W->up[0], W->tail_h, w4(W->up_rb[0]).data(), ws.tail_part, ws.lc_scratch, st));
+            continue;
+        }
+        ConvParams u = conv_base(g[L + 1], nb);
+        u.ntaps = 1; u.off[0] = 0; u.Kt = C[L + 1]; u.N = 4 * C[L]; u.a = ws.a16[L + 1]; u.w = W->up[L];
+        u.mode = 1; u.Cf = C[L]; u.Cf_log2 = 0; while ((1 << u.Cf_log2) < u.Cf) ++u.Cf_log2; u.gf = g[L]; u.gf.M = nb * g[L].S;
+        u.out32 = ws.p32a[L]; u.out16 = ws.a16[L];
+        if (fused) { u.out_lo = ws.lo16[L]; u.out32 = nullptr; }
+        GD_TRY(run_conv(u, prec, st));
+        GD_TRY(resblock(L, W->up_rb[L][0], ws.p32a[L], nullptr, ws.p32b[L], ws.a16[L], nullptr));
+        if (L > 0) {
+            GD_TRY(resblock(L, W->up_rb[L][1], ws.p32b[L], ws.skip32[L], nullptr, ws.a16[L], nullptr));
+        } else if (fused) {             // + x1 enters through the stencil of k_tail_gather; the result only feeds m_tail
+            ConvParams p[2];
+            resblock_params(0, W->up_rb[0][1], ws.p32b[0], nullptr, nullptr, nullptr, nullptr, p);
+            p[1].tail_part = ws.tail_part; p[1].tail_w = W->tail_h;
+            GD_TRY(run_pair(p));
+        } else {
+            GD_TRY(resblock(0, W->up_rb[0][1], ws.p32b[0], ws.skip32[0], ws.p32a[0], nullptr, nullptr));
+        }
+    }
+    // m_tail (ResUNet.py:39): conv(x + x1), times the per-stamp input scale
+    if (chain) return launch_tail_gather(ws.tail_part, 1, g[0], tscale, zout, nb, t, W->tail_head_g, st, 1);
+    if (fused) return launch_tail_gather(ws.tail_part, C[0] / 32, g[0], tscale, zout, nb, ws.tpad, W->tail_head_g, st);
     return launch_tail(ws.p32a[0], W->tail, C[0], g[0], tscale, zout, nb, st);
 }
-
-static int g_fuse_ht_fwd() { return fuse_ht_mode(); }
 
 static int rho_chunk(const GdWeights* W, const Ws& ws, const float* psf, const float* alpha, int nb, cudaStream_t st) {
     if (W->has_subnet) return launch_subnet(W->sub, psf, alpha, ws.rho, nb, st);
@@ -806,11 +684,9 @@ extern "C" int gd_admm_forward(const GdWeights* W, int llh, int u_v0_over_alpha,
             GD_TRY(launch_g_prologue(yc, kc, ac, ws.spec, ws.HtH, ws.z, ws.u, ws.x, nb, st));
             if (n == 0) GD_TRY(copy_f32(out + o, ws.z, ni, st));
             for (int it = 0; it < n; ++it) {
-                const bool xh = xhead_applies(W);
-                if (xh) GD_TRY(launch_g_xupdate(ws.spec, ws.HtH, ws.rho, nr, it, ws.z, ws.x, ws.u, ws.t, ws.tscale, nb, st, W->head_h, &ws.g[0], ws.a16[0], ws.tpad));
-                else GD_TRY(launch_g_xupdate(ws.spec, ws.HtH, ws.rho, nr, it, ws.z, ws.x, ws.u, ws.t, ws.tscale, nb, st));
+                GD_TRY(launch_g_xupdate(ws.spec, ws.HtH, ws.rho, nr, it, ws.z, ws.x, ws.u, ws.t, ws.tscale, nb, st));
                 float* zdst = it == n - 1 ? out + o : ws.z;
-                GD_TRY(resunet_chunk(W, ws, ws.t, ws.tscale, zdst, nb, st, xh));
+                GD_TRY(resunet_chunk(W, ws, ws.t, ws.tscale, zdst, nb, st));
                 if (analysis) {
                     float* A = analysis + (size_t)it * 3 * plane + o;
                     GD_TRY(copy_f32(A, ws.x, ni, st));

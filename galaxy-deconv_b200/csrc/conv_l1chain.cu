@@ -4,8 +4,8 @@
 //   UP:    x  = ResBlock(ResBlock(m_up1's transposed conv of the level-1 map))  -> per-tap m_tail partial sums (k_tail_gather)
 //
 // i.e. FOUR 3x3 convolutions (two `x + conv(ReLU(conv(x)))` blocks, models/resnet_basicblock.py:69-71) per launch with every
-// intermediate on chip.  Why: at this level one conv per launch is HBM-bound (768 MB per 32-channel fp16 map of 5000 stamps) and
-// even the fused ResBlock kernel (conv_rb.cu) moves 3.1 GB per block for 0.3 ms of tensor work.  Here a work item is HALF A
+// intermediate on chip.  Why: at this level one conv per launch is HBM-bound (768 MB per 32-channel fp16 map of 5000 stamps), and
+// even a kernel that runs one whole ResBlock per launch moves 3.1 GB per block for 0.3 ms of tensor work.  Here a work item is HALF A
 // STAMP (24 output rows + the 4 rows of halo the four convs need = a 28-row window, 1372 rows of the padded-linear layout):
 //   * the fp16 operand copies of the stream (X) and of ReLU(conv1) (T) live in shared memory, two buffers of 4 chunk planes
 //     x 1428 rows x 16 B; planes are separated by 56 zero rows that are never written, which serve as the zero row above /

@@ -9,8 +9,6 @@
 #include "kernels.cuh"
 #include "launch.cuh"
 
-#include <cstring>
-
 namespace gd {
 
 constexpr int SIMT_KSLAB = 256;
@@ -110,36 +108,6 @@ __global__ void __launch_bounds__(128) k_head(const float* __restrict__ t, const
     }
 }
 
-// Product-path head for C0 = 32 (tcgen05 path with head/tail fusion): only the fp16 operand copy and the padded-linear copy
-// of the input are written (the fp32 head output is recomputed where it is consumed).  The 288 weights are kernel
-// parameters, i.e. immediate constant-bank operands of the FFMAs -- the generic k_head is bound by its shared-memory loads.
-__global__ void __launch_bounds__(128) k_head32(const float* __restrict__ t, const __grid_constant__ HeadW32 hw, Geom g, __half* __restrict__ out16,
-                                                float* __restrict__ tpad, int batch) {
-    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx >= batch * NPIX) return;
-    const int b = idx / NPIX, r = idx - b * NPIX, y = r / STAMP, x = r - y * STAMP;
-    float in[9];
-#pragma unroll
-    for (int dy = -1; dy <= 1; ++dy)
-#pragma unroll
-        for (int dx = -1; dx <= 1; ++dx) {
-            const int yy = y + dy, xx = x + dx;
-            in[(dy + 1) * 3 + dx + 1] = (yy >= 0 && yy < STAMP && xx >= 0 && xx < STAMP) ? __ldg(t + (size_t)b * NPIX + yy * STAMP + xx) : 0.f;
-        }
-    const int row = g.base0 + b * g.S + y * g.Wp + x;
-    tpad[row] = in[4];
-    float acc[32];
-#pragma unroll
-    for (int c = 0; c < 32; ++c) acc[c] = 0.f;
-#pragma unroll
-    for (int tp = 0; tp < 9; ++tp)
-#pragma unroll
-        for (int c = 0; c < 32; ++c) acc[c] = fmaf(in[tp], hw.w[tp * 32 + c], acc[c]);
-    uint4* dst = reinterpret_cast<uint4*>(out16) + row;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) dst[(size_t)k * g.Ptot] = pack8_half(acc + 8 * k);
-}
-
 // tail: x32 [C0/4][Ptot][4] fp32 -> z [B][48*48] fp32, times the per-stamp power-of-two scale.
 // Works in the padded-linear row space (the halo rows of the stream are zero, so there are no bounds checks): a CTA
 // stages the window rows [m0 - Wp - 1, m0 + TAIL_ROWS + Wp + 1) of all C0/4 planes in shared memory with coalesced
@@ -184,18 +152,16 @@ __global__ void __launch_bounds__(TAIL_ROWS) k_tail(const float* __restrict__ x3
 // times the per-stamp power-of-two input scale.  Since x1 = m_head(t) is linear in the 1-channel input t, its tail is the
 // 81-coefficient composite  tail(x1)[m] = sum_{tap2: m+off2 inside the stamp} sum_tap1 G[tap2][tap1] * t[m + off2 + off1],
 // G = W_tail W_head^T (kernel parameters), evaluated here from the padded-linear copy of t (zero halos) instead of 288 FMAs
-// per row in the conv epilogue.  `G == nullptr-like` (has_g = 0): P already contains x1.  Halo rows of P are never written.
+// per row in the conv epilogue.  Halo rows of P are never written.
 // The zero padding of m_tail drops the taps t2 whose pixel lies outside the stamp, so the composite is one of NINE 5x5 stencils,
 // chosen by whether the pixel sits on the first / last row and column; the host collapses G (81 coefficients) into them.
 struct TailG { float g5[9 * 25]; };
 __global__ void __launch_bounds__(256) k_tail_gather(const float* __restrict__ P, int units, Geom g, const float* __restrict__ tscale,
-                                                     float* __restrict__ z, int batch, const float* __restrict__ tpad, int has_g,
+                                                     float* __restrict__ z, int batch, const float* __restrict__ tpad,
                                                      const __grid_constant__ TailG G, int t_plain) {
     __shared__ float g5s[9 * 25];
-    if (has_g) {
-        if (threadIdx.x < 9 * 25) g5s[threadIdx.x] = G.g5[threadIdx.x];
-        __syncthreads();
-    }
+    if (threadIdx.x < 9 * 25) g5s[threadIdx.x] = G.g5[threadIdx.x];
+    __syncthreads();
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= batch * NPIX) return;
     const int b = idx / NPIX, r = idx - b * NPIX, y = r / STAMP, x = r - y * STAMP;
@@ -206,24 +172,22 @@ __global__ void __launch_bounds__(256) k_tail_gather(const float* __restrict__ P
 #pragma unroll
         for (int t = 0; t < 9; ++t) s += __ldg(src + (size_t)(u * 9 + t) * g.Ptot + (t / 3 - 1) * g.Wp + (t % 3 - 1));
     }
-    if (has_g) {
-        // (a leaner address / predicate computation -- 118 M instead of 199 M warp instructions -- needs 75 registers and is SLOWER,
-        // 262 us against 234 us per 5000 stamps: the kernel is bound by bytes in flight, i.e. by resident threads)
-        const float* c5 = g5s + ((y == 0 ? 0 : y == STAMP - 1 ? 2 : 1) * 3 + (x == 0 ? 0 : x == STAMP - 1 ? 2 : 1)) * 25;
-        float a = 0.f;
+    // (a leaner address / predicate computation -- 118 M instead of 199 M warp instructions -- needs 75 registers and is SLOWER,
+    // 262 us against 234 us per 5000 stamps: the kernel is bound by bytes in flight, i.e. by resident threads)
+    const float* c5 = g5s + ((y == 0 ? 0 : y == STAMP - 1 ? 2 : 1) * 3 + (x == 0 ? 0 : x == STAMP - 1 ? 2 : 1)) * 25;
+    float a = 0.f;
 #pragma unroll
-        for (int dy = -2; dy <= 2; ++dy)
+    for (int dy = -2; dy <= 2; ++dy)
 #pragma unroll
-            for (int dx = -2; dx <= 2; ++dx) {
-                const int yy = y + dy, xx = x + dx;
-                // 5x5 neighbourhood of t (zero outside the stamp).  t_plain: `tpad` is the dense [B][48*48] denoiser input itself
-                // (conv_l1chain.cu path: no padded-linear copy exists)
-                const float tv = (yy >= 0 && yy < STAMP && xx >= 0 && xx < STAMP)
-                                     ? (t_plain ? __ldg(tpad + (size_t)b * NPIX + yy * STAMP + xx) : __ldg(tpad + row + dy * g.Wp + dx)) : 0.f;
-                a = fmaf(c5[(dy + 2) * 5 + dx + 2], tv, a);
-            }
-        s += a;
-    }
+        for (int dx = -2; dx <= 2; ++dx) {
+            const int yy = y + dy, xx = x + dx;
+            // 5x5 neighbourhood of t (zero outside the stamp).  t_plain: `tpad` is the dense [B][48*48] denoiser input itself
+            // (conv_l1chain.cu path: no padded-linear copy exists)
+            const float tv = (yy >= 0 && yy < STAMP && xx >= 0 && xx < STAMP)
+                                 ? (t_plain ? __ldg(tpad + (size_t)b * NPIX + yy * STAMP + xx) : __ldg(tpad + row + dy * g.Wp + dx)) : 0.f;
+            a = fmaf(c5[(dy + 2) * 5 + dx + 2], tv, a);
+        }
+    s += a;
     z[idx] = s * tscale[b];
 }
 
@@ -237,16 +201,9 @@ int launch_conv_simt(const ConvParams& p, int prec, cudaStream_t st) {
     return GD_OK;
 }
 
-int launch_head(const float* t, const float* w, const float* w_host, int C0, const ConvParams& p, int batch, int prec, float* tpad, cudaStream_t st) {
+int launch_head(const float* t, const float* w, int C0, const ConvParams& p, int batch, int prec, float* tpad, cudaStream_t st) {
     int n = batch * NPIX, blocks = (n + 127) / 128;
     if (n <= 0) return GD_OK;
-    if (prec == PREC_FP16_UMMA && C0 == 32 && tpad && !p.out32 && p.out16 && w_host) {
-        HeadW32 hw;
-        memcpy(hw.w, w_host, sizeof(hw.w));
-        k_head32<<<blocks, 128, 0, st>>>(t, hw, p.g, reinterpret_cast<__half*>(p.out16), tpad, batch);
-        GD_LAUNCHED();
-        return GD_OK;
-    }
     if (prec == PREC_FP32_SIMT) k_head<float><<<blocks, 128, 9 * C0 * sizeof(float), st>>>(t, w, C0, p, batch, tpad);
     else k_head<__half><<<blocks, 128, 9 * C0 * sizeof(float), st>>>(t, w, C0, p, batch, tpad);
     GD_LAUNCHED();
@@ -256,23 +213,20 @@ int launch_head(const float* t, const float* w, const float* w_host, int C0, con
 int launch_tail_gather(const float* P, int units, const Geom& g, const float* tscale, float* z, int batch, const float* tpad,
                        const float* G81_host, cudaStream_t st, int t_plain) {
     if (batch <= 0) return GD_OK;
+    // G81[t2 * 9 + t1]: tail tap t2 (pixel p + t2) times head tap t1 (input p + t2 + t1).  Class (cy, cx): 0 = first row / column
+    // (tap -1 falls outside and is dropped), 2 = last, 1 = interior.
+    double acc[9 * 25] = {0};
+    for (int cy = 0; cy < 3; ++cy)
+        for (int cx = 0; cx < 3; ++cx)
+            for (int t2 = 0; t2 < 9; ++t2) {
+                const int ty = t2 / 3, tx = t2 % 3;
+                if ((cy == 0 && ty == 0) || (cy == 2 && ty == 2) || (cx == 0 && tx == 0) || (cx == 2 && tx == 2)) continue;
+                for (int t1 = 0; t1 < 9; ++t1)
+                    acc[(cy * 3 + cx) * 25 + (ty + t1 / 3) * 5 + (tx + t1 % 3)] += (double)G81_host[t2 * 9 + t1];
+            }
     TailG G;
-    memset(&G, 0, sizeof(G));
-    if (G81_host) {
-        // G81[t2 * 9 + t1]: tail tap t2 (pixel p + t2) times head tap t1 (input p + t2 + t1).  Class (cy, cx): 0 = first row / column
-        // (tap -1 falls outside and is dropped), 2 = last, 1 = interior.
-        double acc[9 * 25] = {0};
-        for (int cy = 0; cy < 3; ++cy)
-            for (int cx = 0; cx < 3; ++cx)
-                for (int t2 = 0; t2 < 9; ++t2) {
-                    const int ty = t2 / 3, tx = t2 % 3;
-                    if ((cy == 0 && ty == 0) || (cy == 2 && ty == 2) || (cx == 0 && tx == 0) || (cx == 2 && tx == 2)) continue;
-                    for (int t1 = 0; t1 < 9; ++t1)
-                        acc[(cy * 3 + cx) * 25 + (ty + t1 / 3) * 5 + (tx + t1 % 3)] += (double)G81_host[t2 * 9 + t1];
-                }
-        for (int i = 0; i < 9 * 25; ++i) G.g5[i] = (float)acc[i];
-    }
-    k_tail_gather<<<(batch * NPIX + 255) / 256, 256, 0, st>>>(P, units, g, tscale, z, batch, tpad, G81_host != nullptr, G, t_plain);
+    for (int i = 0; i < 9 * 25; ++i) G.g5[i] = (float)acc[i];
+    k_tail_gather<<<(batch * NPIX + 255) / 256, 256, 0, st>>>(P, units, g, tscale, z, batch, tpad, G, t_plain);
     GD_LAUNCHED();
     return GD_OK;
 }

@@ -469,7 +469,7 @@ int conv_profile_end(double* ms_total, double* flops_total, unsigned long long* 
     return GD_OK;
 }
 
-// Timing hook for the other tcgen05 conv kernels (conv_rb.cu): records the start event and returns the stop event to record.
+// Timing hook for the other tcgen05 conv kernels (conv_l1chain.cu, conv_l2chain.cu): records the start event and returns the stop event to record.
 int conv_profile_mark(double flops, cudaStream_t st, cudaEvent_t* stop) {
     *stop = nullptr;
     if (!g_timing.on) return GD_OK;
@@ -494,7 +494,6 @@ int conv_umma_init() {
     GD_UMMA_ATTR(1, 2); GD_UMMA_ATTR(2, 2); GD_UMMA_ATTR(4, 2); GD_UMMA_ATTR(1, 4); GD_UMMA_ATTR(2, 4); GD_UMMA_ATTR(4, 4);
 #undef GD_UMMA_ATTR
     GD_CUDA_CHECK(cudaFuncSetAttribute(k_conv_umma<2, 2, EPI_HT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UMMA_SMEM_MAX));
-    GD_CUDA_CHECK(cudaFuncSetAttribute(k_conv_umma<4, 2, EPI_HT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UMMA_SMEM_MAX));
     return GD_OK;
 }
 
@@ -514,8 +513,8 @@ static int make_cfg(const ConvParams& p, UmmaCfg* out) {
     c.b_stages = c.b_resident ? 0 : g_bstages;
     size_t b_region = c.b_resident ? (size_t)c.b_total_bytes : (size_t)c.b_stages * c.b_stage_bytes;
     if (p.head_t || p.tail_part) {                // EPI_HT (weights are kernel parameters)
-        if (p.mode != 0 || p.ntaps != 9 || (p.N != 32 && p.N != 64) || p.skip32 || p.s2d || (p.head_t && !p.head_w) || (p.tail_part && !p.tail_w)) {
-            set_error("conv_umma: head/tail fusion needs a 3x3 level-0 layer with N = 32 or 64"); return GD_EUNSUPPORTED;
+        if (p.mode != 0 || p.ntaps != 9 || p.N != 64 || p.skip32 || p.s2d || (p.head_t && !p.head_w) || (p.tail_part && !p.tail_w)) {
+            set_error("conv_umma: head/tail fusion needs a 3x3 level-0 layer with N = 64"); return GD_EUNSUPPORTED;
         }
     } else if (p.mode == 1) {
         c.aux_off = (int)((b_region + 127) / 128 * 128);
@@ -611,7 +610,7 @@ int launch_conv_umma(const ConvParams& p, cudaStream_t st) {
         if (p.tail_part) memcpy(hw.tail, p.tail_w, sizeof(hw.tail));                                \
         k_conv_umma<JJ, KKK, EPI_HT><<<grid, UMMA_THREADS, c.smem, st>>>(p, c, hw);                 \
     } else
-    GD_UMMA_GO_HT(2, 2) GD_UMMA_GO_HT(4, 2)
+    GD_UMMA_GO_HT(2, 2)
     GD_UMMA_GO(1, 2) GD_UMMA_GO(2, 2) GD_UMMA_GO(4, 2) GD_UMMA_GO(1, 4) GD_UMMA_GO(2, 4) GD_UMMA_GO(4, 4)
     { set_error("conv_umma: no kernel variant for J=%d, BK=%d", c.J, c.BK); return GD_EUNSUPPORTED; }
 #undef GD_UMMA_GO

@@ -11,13 +11,11 @@
 // psf_to_otf == roll(N/2) (path U / solvers) are pure phase factors on the spectrum of the image placed at the
 // corner of the grid:  shift by 72 on a 96 grid -> (+i)^(k1+k2), shift by 24 on a 48 grid -> (-1)^(k1+k2).
 #include <math.h>
-#include "conv_epilogue.cuh"
 #include "fft_block.cuh"
 #include "launch.cuh"
 #include "umma_ptx.cuh"
 
 #include <cstdlib>
-#include <cstring>
 #include <mutex>
 #include <vector>
 
@@ -82,17 +80,11 @@ __global__ void __launch_bounds__(G_THREADS) k_g_prologue(const float* __restric
 // iteration `it`:  u <- u + rho_{it-1} (x_prev - z)   (it > 0; the dual update of the previous iteration, :145)
 //                  x <- crop(ifft((Pc + F(rho z - u)) / (rho + HtH)))                                    (:89-93)
 //                  t <- (rho x + u) * 2^-e, tscale = 2^e                                   (denoiser input, :142)
-// HEAD = true (tcgen05 path, C0 = 32, head/tail fusion): the kernel also runs m_head (ResUNet.py:31) on the scaled denoiser
-// input it has just produced -- t goes through shared memory, every thread convolves its 9 pixels (weights = kernel
-// parameters) and writes the fp16 operand copy a16 plus the padded-linear copy tpad -- which saves the k_head32 launch and
-// its re-read of t.
-template <bool HEAD>
 __global__ void __launch_bounds__(G_THREADS) k_g_xupdate(const float2* __restrict__ Pc, const float* __restrict__ HtH,
                                                          const float* __restrict__ rho, int n_rho, int it,
                                                          const float* __restrict__ z, float* __restrict__ x,
                                                          float* __restrict__ u, float* __restrict__ t,
-                                                         float* __restrict__ tscale, const __grid_constant__ HeadW32 hw, const Geom g,
-                                                         __half* __restrict__ a16, float* __restrict__ tpad) {
+                                                         float* __restrict__ tscale) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float2* Z = reinterpret_cast<float2*>(smem_raw);
     float2* S = Z + 24 * 96;
@@ -142,37 +134,6 @@ __global__ void __launch_bounds__(G_THREADS) k_g_xupdate(const float2* __restric
     if (threadIdx.x == 0) tscale[b] = s;
 #pragma unroll
     for (int e = 0; e < PER; ++e) t[o + threadIdx.x + e * G_THREADS] = tv[e] * inv;
-    if constexpr (HEAD) {
-        float* ts = reinterpret_cast<float*>(S);             // the spectrum buffer is free after inv2d
-        __syncthreads();                                      // (every thread is done reading Z / S)
-#pragma unroll
-        for (int e = 0; e < PER; ++e) ts[threadIdx.x + e * G_THREADS] = tv[e] * inv;
-        __syncthreads();
-        for (int e = 0; e < PER; ++e) {
-            const int i = threadIdx.x + e * G_THREADS;
-            const int yy0 = i / STAMP, xx0 = i - yy0 * STAMP;
-            float in[9];
-#pragma unroll
-            for (int dy = -1; dy <= 1; ++dy)
-#pragma unroll
-                for (int dx = -1; dx <= 1; ++dx) {
-                    const int yy = yy0 + dy, xx = xx0 + dx;
-                    in[(dy + 1) * 3 + dx + 1] = (yy >= 0 && yy < STAMP && xx >= 0 && xx < STAMP) ? ts[yy * STAMP + xx] : 0.f;
-                }
-            const int row = g.base0 + b * g.S + yy0 * g.Wp + xx0;
-            tpad[row] = in[4];
-            float acc[32];
-#pragma unroll
-            for (int c = 0; c < 32; ++c) acc[c] = 0.f;
-#pragma unroll
-            for (int tp = 0; tp < 9; ++tp)
-#pragma unroll
-                for (int c = 0; c < 32; ++c) acc[c] = fmaf(in[tp], hw.w[tp * 32 + c], acc[c]);
-            uint4* dst = reinterpret_cast<uint4*>(a16) + row;
-#pragma unroll
-            for (int k = 0; k < 4; ++k) dst[(size_t)k * g.Ptot] = pack8_half(acc + 8 * k);
-        }
-    }
 }
 
 // analysis=True bookkeeping (:147-152): u_i = u + rho_i (x_i - z_i) written to the analysis buffer
@@ -901,8 +862,7 @@ template <class K> static int opt_in_smem(K kernel, size_t bytes) {
 int fft_kernels_init() {
     int rc;
     if ((rc = opt_in_smem(k_g_prologue, G_SMEM_PRO))) return rc;
-    if ((rc = opt_in_smem(k_g_xupdate<false>, G_SMEM_XUP))) return rc;
-    if ((rc = opt_in_smem(k_g_xupdate<true>, G_SMEM_XUP))) return rc;
+    if ((rc = opt_in_smem(k_g_xupdate, G_SMEM_XUP))) return rc;
     if ((rc = opt_in_smem(k_solver, SOLVER_SMEM))) return rc;
     if ((rc = opt_in_smem(k_wiener48, W48_SMEM))) return rc;
     if ((rc = opt_in_smem(k_rl48, W48_SMEM))) return rc;
@@ -922,20 +882,9 @@ int launch_g_prologue(const float* y, const float* psf, const float* alpha, floa
     return GD_OK;
 }
 int launch_g_xupdate(const float2* Pc, const float* HtH, const float* rho, int n_rho, int it, const float* z, float* x,
-                     float* u, float* t, float* tscale, int batch, cudaStream_t st, const float* head_w_host, const Geom* g0,
-                     void* a16, float* tpad) {
+                     float* u, float* t, float* tscale, int batch, cudaStream_t st) {
     if (batch <= 0) return GD_OK;
-    HeadW32 hw;
-    Geom g;
-    memset(&hw, 0, sizeof(hw));
-    memset(&g, 0, sizeof(g));
-    if (head_w_host && g0 && a16 && tpad) {
-        memcpy(hw.w, head_w_host, sizeof(hw.w));
-        k_g_xupdate<true><<<batch, G_THREADS, G_SMEM_XUP, st>>>(Pc, HtH, rho, n_rho, it, z, x, u, t, tscale, hw, *g0,
-                                                              reinterpret_cast<__half*>(a16), tpad);
-    } else {
-        k_g_xupdate<false><<<batch, G_THREADS, G_SMEM_XUP, st>>>(Pc, HtH, rho, n_rho, it, z, x, u, t, tscale, hw, g, nullptr, nullptr);
-    }
+    k_g_xupdate<<<batch, G_THREADS, G_SMEM_XUP, st>>>(Pc, HtH, rho, n_rho, it, z, x, u, t, tscale);
     GD_LAUNCHED();
     return GD_OK;
 }

@@ -58,14 +58,15 @@ GD_HD uint32_t div_by_magic(uint32_t n, uint32_t magic, uint32_t shift) { return
 
 inline Geom make_geom(int H, int batch) {
     Geom g;
-    // base0 >= Wp + 1 zero rows in front of the first stamp; 64 more so that the fused ResBlock kernel (conv_rb.cu), whose
-    // t window starts 64 rows before an item, never reads in front of the buffer
+    // base0 >= Wp + 1 zero rows in front of the first stamp: the A window of k_conv_umma starts Wp + 1 rows before its first tile.
+    // The 64 rows in front of them, like the 5 * MTILE rows at the end of Ptot, are slack that no kernel reads; removing either
+    // would move every buffer offset and change gd_workspace_bytes and gd_max_chunk.
     g.H = H; g.W = H; g.Wp = H + 1; g.S = (H + 1) * (H + 1); g.base0 = g.Wp + 1 + 64;
     div_magic((uint32_t)g.S, &g.magS, &g.shS); div_magic((uint32_t)g.Wp, &g.magW, &g.shW);
     g.M = batch * g.S;
     int mt = ((g.M + MTILE - 1) / MTILE + 7) / 8 * 8;
-    // a CTA of the tcgen05 kernel owns up to 8 consecutive tiles and its window reaches Wp+1 rows past them
-    // (conv_rb.cu: the x window of the last 384-row item ends up to 498 rows past M)
+    // the tiles rounded up to a multiple of 8 hold every work item of k_conv_umma (up to 4 tiles each); the base0 rows after them
+    // hold the Wp + 1 rows its A window reaches past the last item
     g.Ptot = mt * MTILE + 2 * g.base0 + 5 * MTILE;
     return g;
 }
@@ -121,9 +122,6 @@ struct ConvParams {
     float* tail_part;         // [(N/32)*9][g.Ptot] fp32
     const float* tail_w;      // [9][N] fp32, HOST pointer
 };
-
-// fp32 m_head weights [tap][32] passed as a kernel parameter (immediate constant-bank FFMA operands): k_head32, k_g_xupdate
-struct HeadW32 { float w[9 * 32]; };
 
 // ---------------------------------------------------------------------------------------------------
 // error plumbing (C ABI returns ints; message retrievable through gd_last_error())

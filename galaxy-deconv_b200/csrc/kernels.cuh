@@ -13,7 +13,6 @@ int conv_umma_init();
 void conv_profile_begin();
 int conv_profile_end(double* ms_total, double* flops_total, unsigned long long* launches);
 int conv_profile_mark(double flops, cudaStream_t st, cudaEvent_t* stop);
-int conv_rb_init();
 int conv_l1chain_init();
 int launch_l1chain_down(const Geom& g0, const Geom& g1, int nb, const float* t, const float* head_w_host, const void* const* w4, const void* wdown,
                         float* skip32, void* x2_16, void* x2_lo, cudaStream_t st);
@@ -24,14 +23,11 @@ int conv_l2chain_init();
 size_t l2chain_scratch_bytes();
 int launch_l2chain(int mode, const Geom& g1, const Geom& g2, int nb, const void* x_hi, const void* x_lo, const void* const* w4, const void* wdown,
                    float* skip3, void* x3_16, const void* a_coarse, const void* wup, void* scratch, const float* skip32, void* out16, cudaStream_t st);
-bool conv_rb_supported(const ConvParams& p1, const ConvParams& p2);
-int launch_conv_rb(const ConvParams& p1, const ConvParams& p2, cudaStream_t st);
 
 int launch_g_prologue(const float* y, const float* psf, const float* alpha, float2* Pc, float* HtH, float* z, float* u,
                       float* x, int batch, cudaStream_t st);
 int launch_g_xupdate(const float2* Pc, const float* HtH, const float* rho, int n_rho, int it, const float* z, float* x,
-                     float* u, float* t, float* tscale, int batch, cudaStream_t st, const float* head_w_host = nullptr,
-                     const Geom* g0 = nullptr, void* a16 = nullptr, float* tpad = nullptr);
+                     float* u, float* t, float* tscale, int batch, cudaStream_t st);
 int launch_g_dual_out(const float* rho, int n_rho, int it, const float* x, const float* z, const float* u, float* uo,
                       int batch, cudaStream_t st);
 int launch_scale_in(const float* in, float* t, float* tscale, int batch, cudaStream_t st);
@@ -58,7 +54,7 @@ int launch_adaptive_moments(const float* img, int batch, float guess_sigma, floa
 
 int launch_conv_simt(const ConvParams& p, int prec, cudaStream_t st);
 int launch_conv_umma(const ConvParams& p, cudaStream_t st);
-int launch_head(const float* t, const float* w, const float* w_host, int C0, const ConvParams& p, int batch, int prec, float* tpad, cudaStream_t st);
+int launch_head(const float* t, const float* w, int C0, const ConvParams& p, int batch, int prec, float* tpad, cudaStream_t st);
 int launch_tail_gather(const float* P, int units, const Geom& g, const float* tscale, float* z, int batch, const float* tpad,
                        const float* G81_host, cudaStream_t st, int t_plain = 0);
 int launch_tail(const float* x32, const float* w, int C0, const Geom& g, const float* tscale, float* z, int batch,

@@ -1,4 +1,4 @@
-// PTX wrappers shared by the tcgen05 kernels (conv_umma.cu, conv_rb.cu, conv_l1chain.cu): mbarrier, bulk-async copies (TMA engine),
+// PTX wrappers shared by the tcgen05 kernels (conv_umma.cu, conv_l1chain.cu, conv_l2chain.cu): mbarrier, bulk-async copies (TMA engine),
 // tcgen05.mma / commit / ld, shared-memory matrix descriptors.
 #pragma once
 #include <cuda_runtime.h>
@@ -8,7 +8,7 @@
 
 namespace gd {
 
-// ---- kernel shape constants shared by conv_umma.cu and conv_rb.cu ----
+// ---- kernel shape constants of conv_umma.cu (the chain kernels also allocate TMEM_COLS) ----
 enum { EPI_PLAIN = 0, EPI_FULL = 1, EPI_HT = 2 };   // EPI_HT = EPI_FULL + head recompute / tail partial sums (level 0)
 constexpr int EPI_WARPS = 8;
 constexpr int MMA_WARPS = 4;                        // warps 1..4: MMA issuers, one 128-row tile of the item each (J <= 4)

@@ -1,6 +1,6 @@
 #!/bin/bash
 # Fast iteration pass: GPU tests, headline bench (optionally under A/B environment switches given as arguments, e.g.
-# "GDECONV_FUSE_HT=0"), and the per-layer ncu table of one denoiser call.
+# "GDECONV_CLUSTER=1"), and the per-layer ncu table of one denoiser call.
 #   gpurun --timeout 1200 -- 'bash tools/gpu/iter.sh [ENV=VAL ...]'
 mkdir -p gpurun_out
 timeout 900 python -m pytest tests -q -m gpu -x --tb=short > gpurun_out/t_gpu.log 2>&1; echo "pytest rc=$?"; tail -n 15 gpurun_out/t_gpu.log

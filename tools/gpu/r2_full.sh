@@ -5,4 +5,3 @@ timeout 1500 python -m pytest tests -q -m gpu -x --tb=short > gpurun_out/t_gpu.l
 timeout 400 python bench.py --steps 5 --warmup 3 > gpurun_out/b_full.json 2> gpurun_out/b1.err; echo "bench rc=$?"; cut -c1-900 gpurun_out/b_full.json; tail -3 gpurun_out/b1.err
 timeout 300 python tools/bench_configs.py > gpurun_out/configs12.jsonl 2>&1; cut -c1-220 gpurun_out/configs12.jsonl
 timeout 600 python tools/parity_report.py 48 > gpurun_out/parity_r02.md 2> gpurun_out/parity.err; echo "parity rc=$?"; cat gpurun_out/parity_r02.md
-GDECONV_L1CHAIN=0 timeout 300 python tools/parity_report.py 48 2>/dev/null | grep "subnet=False" > gpurun_out/parity_r02_nochain.md; cat gpurun_out/parity_r02_nochain.md
