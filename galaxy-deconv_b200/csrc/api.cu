@@ -184,6 +184,7 @@ static int init_once(int device) {
     GD_TRY(conv_l1chain_init());
     GD_TRY(conv_l2chain_init());
     GD_TRY(synth_init());
+    GD_TRY(fpfs_init());
     done.fetch_or(1u << device);
     return GD_OK;
 }
@@ -805,6 +806,22 @@ extern "C" int gd_adaptive_moments(const float* img, int batch, float guess_sigm
     GD_CUDA_CHECK(cudaGetDevice(&dev));
     GD_TRY(init_once(dev));
     return launch_adaptive_moments(img, batch, guess_sigma, shape, info, (cudaStream_t)stream);
+}
+
+extern "C" int gd_fpfs(const float* img, const float* psf, int psf_batch, int batch, float sigma, float cnst, float* modes, float* ell,
+                       void* stream) {
+    if (batch < 0) GD_FAIL(GD_EBADSHAPE, "gd_fpfs: batch %d < 0", batch);
+    if (batch && (!img || !ell)) GD_FAIL(GD_EBADSHAPE, "gd_fpfs: NULL img or ell for a batch of %d", batch);
+    if (psf ? !(psf_batch == 1 || (psf_batch == batch && batch > 0)) : psf_batch != 0)
+        GD_FAIL(GD_EBADSHAPE, "gd_fpfs: psf_batch %d with %s psf for a batch of %d (NULL psf <=> 0; otherwise 1 or the batch)", psf_batch,
+                psf ? "a" : "a NULL", batch);
+    if (!(sigma > 0.f && sigma <= 24.f)) GD_FAIL(GD_EBADSHAPE, "gd_fpfs: sigma must be in (0, 24] px, got %g", (double)sigma);
+    if (!(isfinite(cnst) && cnst >= 0.f)) GD_FAIL(GD_EBADSHAPE, "gd_fpfs: const must be finite and >= 0, got %g", (double)cnst);
+    if (batch == 0) return GD_OK;
+    int dev;
+    GD_CUDA_CHECK(cudaGetDevice(&dev));
+    GD_TRY(init_once(dev));
+    return launch_fpfs(img, psf, psf_batch, batch, sigma, cnst, modes, ell, (cudaStream_t)stream);
 }
 
 extern "C" int gd_debug_geom(int H, int batch, int* geom7) {

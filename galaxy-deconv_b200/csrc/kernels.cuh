@@ -1,5 +1,5 @@
 // Host-callable launchers of every kernel in libgdeconv (definitions in fft_kernels.cu, subnet.cu, conv_simt.cu,
-// conv_umma.cu, synth.cu, shape.cu).  All are stream-ordered and return GD_OK or a negative GD_E* code.
+// conv_umma.cu, synth.cu, shape.cu, fpfs.cu).  All are stream-ordered and return GD_OK or a negative GD_E* code.
 #pragma once
 #include "gd_common.cuh"
 #include "subnet.cuh"
@@ -51,6 +51,9 @@ int synth_init();
 int launch_synth(int64_t start, int count, int64_t seed, int mixed, float snr, float fwhm_err, float shear_err, float* obs,
                  float* psf, float* alpha, float* gt, cudaStream_t st);
 int launch_adaptive_moments(const float* img, int batch, float guess_sigma, float* shape, int32_t* info, cudaStream_t st);
+int fpfs_init();
+int launch_fpfs(const float* img, const float* psf, int psf_batch, int batch, float sigma, float cnst, float* modes, float* ell,
+                cudaStream_t st);
 
 int launch_conv_simt(const ConvParams& p, int prec, cudaStream_t st);
 int launch_conv_umma(const ConvParams& p, cudaStream_t st);

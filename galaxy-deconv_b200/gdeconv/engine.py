@@ -540,6 +540,34 @@ def adaptive_moments(img, guess_sigma=3.0):
     return dict(flux=shape[:, 0], centroid=shape[:, 1:3], M=M, e=shape[:, 6:8], sigma=sigma, status=info[:, 0], n_iter=info[:, 1])
 
 
+def fpfs(img, psf=None, sigma=3.5, const=0.0):
+    """FPFS shear estimation of every stamp (gd_fpfs, csrc/fpfs.cu; the estimator behind the reference's `estimate_shear`,
+    built from Li, Li & Mandelbaum 2018 without bit parity with the fpfs package): the power spectrum of ``img``, divided by the
+    normalised PSF power of ``psf`` (None: a delta PSF), projected on shapelet modes of scale ``sigma`` px.  ``img`` is fp32
+    CUDA [B,1,48,48], ``psf`` None, [1,1,48,48] or [B,1,48,48] on the same device (its normalisation and centring do not
+    matter); ``const`` >= 0 is added to M00 in the denominators.  The work runs on the current stream of img's device.
+    Returns a dict: modes [B,6] (M00, M22c, M22s, M40, M42c, M42s), e [B,2], R [B] (the shear response) and g [B,2] = e / R,
+    the per-galaxy shear; the ensemble shear is e.sum(0) / R.sum()."""
+    img = require_cuda_stamps('img', img)
+    B, dev = img.shape[0], img.device
+    if psf is not None:
+        if torch.is_tensor(psf) and psf.is_cuda and psf.device != dev:
+            raise ValueError(f'psf is on {psf.device}, img on {dev}')
+        psf = require_cuda_stamps('psf', psf)
+        if psf.shape[0] not in (1, B):
+            raise ValueError(f'psf must have batch 1 or {B}, got {psf.shape[0]}')
+        if B == 0:
+            psf = None
+    modes = torch.empty(B, 6, device=dev)
+    ell = torch.empty(B, 3, device=dev)
+    with torch.cuda.device(dev):
+        check(lib.gd_fpfs(_ptr(img), _ptr(psf), 0 if psf is None else psf.shape[0], B, float(sigma), float(const), _ptr(modes),
+                          _ptr(ell), _stream(dev)))
+        e, R = ell[:, :2], ell[:, 2]
+        g = e / R[:, None]
+    return dict(modes=modes, e=e, R=R, g=g)
+
+
 def synth_batch(device, start, count, seed, snr_mode, snr, psf_fwhm_err, psf_shear_err, obs=None, psf=None, alpha=None, gt=None):
     """gd_synth_batch on `device`'s current stream into preallocated contiguous fp32 CUDA tensors (any may be None, not all)."""
     with torch.cuda.device(device):

@@ -177,6 +177,26 @@ GD_API int gd_synth_batch(int64_t start, int count, int64_t seed, int snr_mode, 
 enum { GD_SHAPE_OK = 0, GD_SHAPE_MAXITER = 1, GD_SHAPE_FLUX = 2, GD_SHAPE_MOMENTS = 3, GD_SHAPE_CENTROID = 4 };
 GD_API int gd_adaptive_moments(const float* img, int batch, float guess_sigma, float* shape, int32_t* info, void* stream);
 
+/* FPFS shear estimation (Li, Li & Mandelbaum 2018, MNRAS 481, 4445): the estimator the reference's evaluation runs every stamp
+ * through (utils/utils_test.py:33-49, `estimate_shear` of the fpfs package), built from its definition; bit parity with fpfs
+ * 3.0.2 is not claimed, and its noise-bias correction is not applied.  Pixel p = 48 r + c is at x = c, y = r.  On the grid
+ * k = 2 pi (u, v) / 48 (u, v the fftfreq integers -24..23, kx along columns) with r^2 = sigma^2 |k|^2, G = exp(-r^2/2),
+ * cos2phi = (kx^2 - ky^2)/|k|^2 and sin2phi = 2 kx ky/|k|^2 (both 0 at k = 0), the deconvolved power
+ * D = |I~(k)|^2 / P(k), I~ = sum_x I(x) exp(-i k.x), P = |p~(k)|^2 / |p~(0)|^2 (cells with P < 1e-8 give 0; psf NULL: P = 1,
+ * a delta PSF) gives, summed over all 2304 cells,
+ *   M00  = 1/(sigma sqrt(pi)) sum D G,               M22c, M22s = 1/(sigma sqrt(2 pi)) sum D r^2 (cos2phi, sin2phi) G,
+ *   M40  = 1/(sigma sqrt(pi)) sum D (r^4 - 4 r^2 + 2)/2 G,   M42c, M42s = -1/(sigma sqrt(6 pi)) sum D r^2 (3 - r^2) (cos2phi, sin2phi) G;
+ * with w = M00 + cnst: e1 = -M22c/w, e2 = -M22s/w (e1 > 0 for a galaxy elongated along x), e41 = -M42c/w, e42 = -M42s/w and the
+ * response R = (M00 - M40)/(sqrt(2) w) + sqrt(6)/2 (e1 e41 + e2 e42).  The shear of one galaxy is (e1, e2) / R, of an ensemble
+ * sum e / sum R.
+ *   img    [batch][48*48] fp32 device;  psf [psf_batch][48*48] fp32 device, psf_batch 1 (one PSF for all) or batch; NULL <=> psf_batch 0
+ *   sigma  weight scale in (0, 24] px (3.5 keeps G / P below ~1.6 for PSFs of FWHM <= 4.75 px);  cnst >= 0, finite, in M00's units
+ *   modes  [batch][6] fp32 device (M00, M22c, M22s, M40, M42c, M42s) or NULL;  ell [batch][3] fp32 device (e1, e2, R)
+ * e1, e2, R are NaN where w <= 0 (an all-zero stamp with cnst = 0); all nine outputs are NaN for a stamp whose PSF does not sum
+ * to a positive value.  A stamp's result does not depend on the batch it is measured in. */
+GD_API int gd_fpfs(const float* img, const float* psf, int psf_batch, int batch, float sigma, float cnst, float* modes, float* ell,
+                   void* stream);
+
 /* Test hook: one tap-GEMM layer of the denoiser on caller-packed operands (layouts of csrc/gd_common.cuh:
  * activations [Kt/CH][Ptot][CH], CH = 8 halves (fp16 modes) or 4 floats; weights as gd_pack_weights lays them out
  * for `precision`; out32 [N/4][Ptot][4] fp32).  ntaps = 9 (3x3, zero padding) or 1.  `geom7` receives
