@@ -1,5 +1,5 @@
 // Host-callable launchers of every kernel in libgdeconv (definitions in fft_kernels.cu, subnet.cu, conv_simt.cu,
-// conv_umma.cu, synth.cu, shape.cu, fpfs.cu).  All are stream-ordered and return GD_OK or a negative GD_E* code.
+// conv_umma.cu, synth.cu, shape.cu, fpfs.cu, metacal.cu).  All are stream-ordered and return GD_OK or a negative GD_E* code.
 #pragma once
 #include "gd_common.cuh"
 #include "subnet.cuh"
@@ -54,6 +54,9 @@ int launch_adaptive_moments(const float* img, int batch, float guess_sigma, floa
 int fpfs_init();
 int launch_fpfs(const float* img, const float* psf, int psf_batch, int batch, float sigma, float cnst, float* modes, float* ell,
                 cudaStream_t st);
+int metacal_init();
+int launch_metacal(const float* img, const float* psf, int psf_batch, int batch, float delta, float sigma, float guess_sigma,
+                   float* images, float* shape, int32_t* info, cudaStream_t st);
 
 int launch_conv_simt(const ConvParams& p, int prec, cudaStream_t st);
 int launch_conv_umma(const ConvParams& p, cudaStream_t st);

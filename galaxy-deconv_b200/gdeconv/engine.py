@@ -568,6 +568,45 @@ def fpfs(img, psf=None, sigma=3.5, const=0.0):
     return dict(modes=modes, e=e, R=R, g=g)
 
 
+def metacal(img, psf=None, delta=0.01, reconv_sigma=2.5, guess_sigma=3.0, images=False):
+    """Metacalibration of every stamp (gd_metacal, csrc/metacal.cu): ``img`` deconvolved by ``psf`` (None: no deconvolution, for
+    stamps that are already deconvolved), sheared by (0,0), (+delta,0), (-delta,0), (0,+delta), (0,-delta), reconvolved with a
+    round Gaussian of sigma ``reconv_sigma`` px (one for the whole call) and measured with adaptive moments started at
+    ``guess_sigma`` px.  ``img`` is fp32 CUDA [B,1,48,48], ``psf`` None, [1,1,48,48] or [B,1,48,48] on the same device (its
+    normalisation does not matter; it is centred on pixel (24, 24)).  The work runs on the current stream of img's device.
+    Returns a dict: e [B,5,2] and status, n_iter [B,5] int32 (_lib.SHAPE_*) of the five images in that order, the response
+    R [B,2,2] with R[:, i, j] = (e_i(+delta_j) - e_i(-delta_j)) / (2 delta), the per-galaxy shear g [B,2] = R^-1 e(noshear) (NaN
+    unless all five statuses are OK) and, with ``images=True``, the five images [B,5,1,48,48].  The shear of an ensemble is
+    mean(R)^-1 mean(e(noshear)) over the stamps whose five statuses are OK."""
+    img = require_cuda_stamps('img', img)
+    B, dev = img.shape[0], img.device
+    if psf is not None:
+        if torch.is_tensor(psf) and psf.is_cuda and psf.device != dev:
+            raise ValueError(f'psf is on {psf.device}, img on {dev}')
+        psf = require_cuda_stamps('psf', psf)
+        if psf.shape[0] not in (1, B):
+            raise ValueError(f'psf must have batch 1 or {B}, got {psf.shape[0]}')
+        if B == 0:
+            psf = None
+    ims = torch.empty(B, 5, 1, STAMP, STAMP, device=dev) if images else None
+    shape = torch.empty(B, 5, 8, device=dev)
+    info = torch.empty(B, 5, 2, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        if B:
+            check(lib.gd_metacal(_ptr(img), _ptr(psf), 0 if psf is None else psf.shape[0], B, float(delta), float(reconv_sigma),
+                                 float(guess_sigma), _ptr(ims), _ptr(shape), _ptr(info), _stream(dev)))
+        e, status = shape[:, :, 6:8], info[:, :, 0]
+        R = torch.stack([e[:, 1] - e[:, 2], e[:, 3] - e[:, 4]], 2) / (2 * float(delta))
+        det = R[:, 0, 0] * R[:, 1, 1] - R[:, 0, 1] * R[:, 1, 0]
+        e0 = e[:, 0]
+        g = torch.stack([R[:, 1, 1] * e0[:, 0] - R[:, 0, 1] * e0[:, 1], R[:, 0, 0] * e0[:, 1] - R[:, 1, 0] * e0[:, 0]], 1) / det[:, None]
+        g = torch.where((status == _lib.SHAPE_OK).all(1)[:, None], g, torch.full_like(g, float('nan')))
+    out = dict(e=e, status=status, n_iter=info[:, :, 1], R=R, g=g)
+    if images:
+        out['images'] = ims
+    return out
+
+
 def synth_batch(device, start, count, seed, snr_mode, snr, psf_fwhm_err, psf_shear_err, obs=None, psf=None, alpha=None, gt=None):
     """gd_synth_batch on `device`'s current stream into preallocated contiguous fp32 CUDA tensors (any may be None, not all)."""
     with torch.cuda.device(device):

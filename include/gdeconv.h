@@ -197,6 +197,23 @@ GD_API int gd_adaptive_moments(const float* img, int batch, float guess_sigma, f
 GD_API int gd_fpfs(const float* img, const float* psf, int psf_batch, int batch, float sigma, float cnst, float* modes, float* ell,
                    void* stream);
 
+/* Metacalibration (Huff & Mandelbaum 2017; Sheldon & Huff 2017): each stamp deconvolved by its PSF, sheared by +-delta along
+ * each component, reconvolved with a round Gaussian of sigma reconv_sigma px and measured with gd_adaptive_moments' estimator.
+ * Pixel p = 48 r + c is at X = c - 24, Y = r - 24; on the grid k = 2 pi (u, v) / 48 (u, v the fftfreq integers -24..23, kx along
+ * columns), with I~(q) = sum I[r,c] exp(-i (qx X + qy Y)), A_g = [[1+g1, g2], [g2, 1-g1]] / sqrt(1 - g1^2 - g2^2) and
+ * G~(k) = exp(-reconv_sigma^2 |k|^2 / 2), image j of the shears (0,0), (+d,0), (-d,0), (0,+d), (0,-d) (noshear, 1p, 1m, 2p, 2m) is
+ *   Re ifft2(M_j (-1)^(u+v)),   M_j(k) = I~(A_j k) G~(k) / P(A_j k),   P = p~ / p~(0)
+ * with M_j = 0 where |P|^2 < 1e-8 and on the Nyquist row and column (psf NULL: P = 1).  The response is
+ * R[i][j] = (e_i(+d_j) - e_i(-d_j)) / (2 d) and the shear g = R^-1 e(noshear); of an ensemble, <R>^-1 <e(noshear)> over the stamps
+ * whose five statuses are GD_SHAPE_OK.  No noise-bias ("fix-noise") correction.
+ *   img    [batch][48*48] fp32 device;  psf [psf_batch][48*48] fp32 device, psf_batch 1 (one PSF for all) or batch; NULL <=> psf_batch 0
+ *   delta  in (0, 0.1];  reconv_sigma, guess_sigma (the adaptive-moments start) finite, in (0, 24] px
+ *   images [batch][5][48*48] fp32 device or NULL;  shape [batch][5][8] fp32 device, gd_adaptive_moments' record of each image;
+ *   info   [batch][5][2] int32 device (status GD_SHAPE_*, passes).  shape and info must not be NULL.
+ * A stamp's result does not depend on the batch it is measured in, nor on whether its PSF is given once or repeated. */
+GD_API int gd_metacal(const float* img, const float* psf, int psf_batch, int batch, float delta, float reconv_sigma, float guess_sigma,
+                      float* images, float* shape, int32_t* info, void* stream);
+
 /* Test hook: one tap-GEMM layer of the denoiser on caller-packed operands (layouts of csrc/gd_common.cuh:
  * activations [Kt/CH][Ptot][CH], CH = 8 halves (fp16 modes) or 4 floats; weights as gd_pack_weights lays them out
  * for `precision`; out32 [N/4][Ptot][4] fp32).  ntaps = 9 (3x3, zero padding) or 1.  `geom7` receives
