@@ -186,6 +186,7 @@ static int init_once(int device) {
     GD_TRY(synth_init());
     GD_TRY(fpfs_init());
     GD_TRY(metacal_init());
+    GD_TRY(metacal_fixnoise_init());
     done.fetch_or(1u << device);
     return GD_OK;
 }
@@ -843,6 +844,34 @@ extern "C" int gd_metacal(const float* img, const float* psf, int psf_batch, int
     GD_CUDA_CHECK(cudaGetDevice(&dev));
     GD_TRY(init_once(dev));
     return launch_metacal(img, psf, psf_batch, batch, delta, reconv_sigma, guess_sigma, images, shape, info, (cudaStream_t)stream);
+}
+
+extern "C" int gd_metacal_fixnoise(const float* img, const float* psf, int psf_batch, int batch, float delta, float reconv_sigma,
+                                   float guess_sigma, const float* noise, const float* noise_sigma, int sigma_batch, int64_t start,
+                                   int64_t seed, float* images, float* shape, int32_t* info, void* stream) {
+    if (batch < 0) GD_FAIL(GD_EBADSHAPE, "gd_metacal_fixnoise: batch %d < 0", batch);
+    if (!shape || !info) GD_FAIL(GD_EBADSHAPE, "gd_metacal_fixnoise: NULL shape or info");
+    if (batch && !img) GD_FAIL(GD_EBADSHAPE, "gd_metacal_fixnoise: NULL img for a batch of %d", batch);
+    if (psf ? !(psf_batch == 1 || (psf_batch == batch && batch > 0)) : psf_batch != 0)
+        GD_FAIL(GD_EBADSHAPE, "gd_metacal_fixnoise: psf_batch %d with %s psf for a batch of %d (NULL psf <=> 0; otherwise 1 or the batch)",
+                psf_batch, psf ? "a" : "a NULL", batch);
+    if (!(delta > 0.f && delta <= 0.1f)) GD_FAIL(GD_EBADSHAPE, "gd_metacal_fixnoise: delta must be in (0, 0.1], got %g", (double)delta);
+    if (!(isfinite(reconv_sigma) && reconv_sigma > 0.f && reconv_sigma <= 24.f))
+        GD_FAIL(GD_EBADSHAPE, "gd_metacal_fixnoise: reconv_sigma must be finite and in (0, 24] px, got %g", (double)reconv_sigma);
+    if (!(isfinite(guess_sigma) && guess_sigma > 0.f && guess_sigma <= 24.f))
+        GD_FAIL(GD_EBADSHAPE, "gd_metacal_fixnoise: guess_sigma must be finite and in (0, 24] px, got %g", (double)guess_sigma);
+    if (!noise == !noise_sigma) GD_FAIL(GD_EBADSHAPE, "gd_metacal_fixnoise: exactly one of noise and noise_sigma must be given");
+    if (noise_sigma ? !(sigma_batch == 1 || (sigma_batch == batch && batch > 0)) : sigma_batch != 0)
+        GD_FAIL(GD_EBADSHAPE, "gd_metacal_fixnoise: sigma_batch %d with %s noise_sigma for a batch of %d (NULL <=> 0; otherwise 1 or the batch)",
+                sigma_batch, noise_sigma ? "a" : "a NULL", batch);
+    if (start < 0 || start > INT64_MAX - batch)
+        GD_FAIL(GD_EBADSHAPE, "gd_metacal_fixnoise: stamp range [%lld, +%d) out of range", (long long)start, batch);
+    if (batch == 0) return GD_OK;
+    int dev;
+    GD_CUDA_CHECK(cudaGetDevice(&dev));
+    GD_TRY(init_once(dev));
+    return launch_metacal_fixnoise(img, psf, psf_batch, batch, delta, reconv_sigma, guess_sigma, noise, noise_sigma, sigma_batch, start, seed,
+                                   images, shape, info, (cudaStream_t)stream);
 }
 
 extern "C" int gd_debug_geom(int H, int batch, int* geom7) {

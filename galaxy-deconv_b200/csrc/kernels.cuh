@@ -1,5 +1,5 @@
 // Host-callable launchers of every kernel in libgdeconv (definitions in fft_kernels.cu, subnet.cu, conv_simt.cu,
-// conv_umma.cu, synth.cu, shape.cu, fpfs.cu, metacal.cu).  All are stream-ordered and return GD_OK or a negative GD_E* code.
+// conv_umma.cu, synth.cu, shape.cu, fpfs.cu, metacal.cu, metacal_fixnoise.cu).  All are stream-ordered and return GD_OK or a negative GD_E* code.
 #pragma once
 #include "gd_common.cuh"
 #include "subnet.cuh"
@@ -57,6 +57,10 @@ int launch_fpfs(const float* img, const float* psf, int psf_batch, int batch, fl
 int metacal_init();
 int launch_metacal(const float* img, const float* psf, int psf_batch, int batch, float delta, float sigma, float guess_sigma,
                    float* images, float* shape, int32_t* info, cudaStream_t st);
+int metacal_fixnoise_init();
+int launch_metacal_fixnoise(const float* img, const float* psf, int psf_batch, int batch, float delta, float sigma, float guess_sigma,
+                            const float* noise, const float* noise_sigma, int sigma_batch, int64_t start, int64_t seed, float* images,
+                            float* shape, int32_t* info, cudaStream_t st);
 
 int launch_conv_simt(const ConvParams& p, int prec, cudaStream_t st);
 int launch_conv_umma(const ConvParams& p, cudaStream_t st);

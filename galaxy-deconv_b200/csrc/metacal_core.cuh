@@ -12,11 +12,32 @@
 // from the FFT (Fft48 column and row passes, as k_fpfs); the four sheared ones are off the grid and come from the direct DTFT
 // (dtft below).  The spectra live in "planes" of 24 rows (v = 0..23; the Nyquist row is zero) of PROW float2, fft column order.
 //
-// k_metacal (metacal.cu) and the host test tests/cpu/test_metacal_core.cpp run this code.
+// Fix-noise (Sheldon & Huff 2017).  Metacalibration shears the stamp's noise with the galaxy, and adaptive moments respond to the
+// sheared noise as to a shear.  With a second noise field n of the stamp's kind, fix-noise image j is
+//   T_j(I) + rot^-1(T_j(rot n))
+// where T_j maps a stamp to image j above (deconvolution, shear, reconvolution, floor, Nyquist rule and centring) and
+// rot(a)[r][c] = a[c][47 - r] (numpy's rot90).  A quarter turn flips the sign of a shear, so the two noise fields are sheared in
+// opposite senses and their spurious responses cancel; the images carry twice the noise variance of the stamp.  The second term
+// folds into plane j:
+//   rot(a)(X, Y) = a(-Y - 1, X), so FT[rot a](q) = exp(i qy) a~(R q) and, on the grid, FT[rot^-1 m](k) = exp(i kx) m~(R^-1 k),
+//   with R (x, y) = (-y, x).  With R A_g R^-1 = A_-g and F_j(k) = G~(k) / P(A_j k) (G~ without a PSF; 0 where floored and on the
+//   Nyquist row and column):
+//     FT[rot^-1 T_j rot n](k) = exp(i (kx + qy)) n~(A_j' k) F_j(R^-1 k),   q = A_j R^-1 k
+//   j' is the opposite shear (1p <-> 1m, 2p <-> 2m, noshear <-> noshear).  For noshear qy = -kx: the phase is 1.  R^-1 (u, v) =
+//   (v, -u) maps the grid onto itself and the Nyquist row and column onto each other, so F_j(R^-1 k) of a target is the factor
+//   of another target, or the conjugate of its mirror (F_j(-k) = conj F_j(k)); G~ is unchanged by it.
+// So fix-noise needs one more DTFT per (shear, target), of n at A_j' k (noshear: at k), and no more planes or factors.  The
+// generated field of stamp idx is n[p] = sigma N(idx, p), gdsynth._hashed_normal on streams 60 / 61 (gdsynth's draws use streams
+// 10-51, so it is independent of the obs noise under any seed).
+//
+// k_metacal (metacal.cu), k_metacal_fixnoise (metacal_fixnoise.cu) and the host tests tests/cpu/test_metacal_core.cpp and
+// tests/cpu/test_metacal_fixnoise_core.cpp run this code.
 #pragma once
 #include <cuda_runtime.h>
 #include <math.h>
+#include <stdint.h>
 #include "fft_core.cuh"
+#include "synth_core.cuh"
 
 #ifndef GD_HD
 #define GD_HD __host__ __device__ __forceinline__
@@ -202,6 +223,45 @@ GD_HD void inv_col_store(const float2 (&x)[STAMP], int c, float* img) {
         img[r * STAMP + c] = p.x * S;
         img[r * STAMP + c + HALF] = -p.y * S;
     }
+}
+
+// ---- fix-noise ----
+constexpr int FIXNOISE_STREAM = 60;              // streams 60 / 61
+
+// pixel p of the generated fix-noise field of stamp idx: sigma N(idx, p); a non-finite sigma gives NaN (the stamp fails)
+GD_HD float fixnoise_pixel(uint64_t idx, int p, uint64_t seed, float sigma) {
+    return isfinite(sigma) ? gdsyn::fmul(sigma, gdsyn::hashed_normal(idx, p, seed, FIXNOISE_STREAM)) : NAN;
+}
+
+// the opposite shear j' of shear j: 1p <-> 1m, 2p <-> 2m, noshear itself
+GD_HD int opposite(int j) { return j ? ((j & 1) ? j + 1 : j - 1) : 0; }
+
+// the target whose factor is F_j(R^-1 k) for the target cell (v, u), R^-1 (u, v) = (v, -u): for u <= 0 the cell (v, -u) itself;
+// for u > 0 it lies in the lower half plane and the target is its mirror (-v, u), whose factor is conjugated
+struct RotTarget { int t; bool conj; };
+GD_HD RotTarget rotated_target(int v, int u) {
+    if (u <= 0) return {u == 0 ? v : HALF + (-u - 1) * (STAMP - 1) + v, false};
+    return {HALF + (u - 1) * (STAMP - 1) + (v ? STAMP - 1 - v : 0), true};
+}
+
+// exp(i (kx + qy)), q = A_j R^-1 k, of the cell (v, u)
+GD_HD float2 rotation_phase(int j, float delta, int u, int v) {
+    const float2 q = sheared_freq(j, delta, v, -u);
+    return expi_turns(-((float)u + q.y) * (1.0f / STAMP));
+}
+
+// the fix-noise term of target t of plane j: sgn exp(i (kx + qy)) n~(A_j' k) F_j(R^-1 k), with nt = n~(A_j' k) (centred);
+// factor: the PSF's table [5][1105], or NULL (no PSF: F_j(R^-1 k) = G~(k))
+GD_HD float2 fixnoise_value(int j, int t, float delta, float sigma, float2 nt, const float2* factor) {
+    const Cell k = target(t);
+    const int u = fftfreq(k.i);
+    const float sgn = centre_sign(k.v, k.i);
+    if (j) nt = gdfft::cmul(nt, rotation_phase(j, delta, u, k.v));
+    if (!factor) return cell_value(nt, reconv(k.v, k.i, sigma), sgn);
+    const RotTarget r = rotated_target(k.v, u);
+    float2 f = factor[j * NTARGET + r.t];
+    if (r.conj) f.y = -f.y;
+    return cell_value(nt, f, sgn);
 }
 
 }  // namespace gdmetacal

@@ -79,11 +79,11 @@ GD_HD float hashed_uniform(uint64_t idx, int stream, uint64_t seed) {
     return (float)(uint32_t)(x >> 40) * (1.0f / 16777216.0f);
 }
 
-// standard normal for noise key idx*4099 + j (gdsynth._hashed_normal, streams 40 / 41)
-GD_HD float hashed_normal(uint64_t idx, int j, uint64_t seed) {
+// standard normal for noise key idx*4099 + j (gdsynth._hashed_normal on streams stream0 / stream0 + 1; obs noise: 40 / 41)
+GD_HD float hashed_normal(uint64_t idx, int j, uint64_t seed, int stream0 = 40) {
     const uint64_t key = idx * 4099ull + (uint64_t)j;
-    const float u1 = fmaxf(hashed_uniform(key, 40, seed), 1.0f / 16777216.0f);
-    const float u2 = hashed_uniform(key, 41, seed);
+    const float u1 = fmaxf(hashed_uniform(key, stream0, seed), 1.0f / 16777216.0f);
+    const float u2 = hashed_uniform(key, stream0 + 1, seed);
     return fmul(sqrtf(fmul(-2.0f, logf(u1))), cosf(fmul(TWO_PI_F, u2)));
 }
 

@@ -23,7 +23,7 @@ SYMBOLS = ('gd_version', 'gd_last_error', 'gd_pack_weights', 'gd_free_weights', 
            'gd_admm_forward', 'gd_resunet_forward', 'gd_subnet_forward', 'gd_fft_solver', 'gd_conv_fft', 'gd_moments_e',
            'gd_launch_count', 'gd_debug_geom', 'gd_debug_tapgemm', 'gd_profile_begin', 'gd_profile_end', 'gd_pack_xdense', 'gd_free_xdense', 'gd_xdense_workspace_bytes',
            'gd_xdense_forward', 'gd_tikhonet_forward', 'gd_admm_forward_xdense', 'gd_psf_to_otf', 'gd_conv_otf', 'gd_max_chunk', 'gd_debug_divmagic', 'gd_synth_batch',
-           'gd_adaptive_moments', 'gd_fpfs', 'gd_metacal')
+           'gd_adaptive_moments', 'gd_fpfs', 'gd_metacal', 'gd_metacal_fixnoise')
 
 
 class GdTensorDesc(C.Structure):
@@ -74,6 +74,7 @@ def _load():
     lib.gd_adaptive_moments.argtypes = [vp, i, f, vp, vp, vp]
     lib.gd_fpfs.argtypes = [vp, vp, i, i, f, f, vp, vp, vp]
     lib.gd_metacal.argtypes = [vp, vp, i, i, f, f, f, vp, vp, vp, vp]
+    lib.gd_metacal_fixnoise.argtypes = [vp, vp, i, i, f, f, f, vp, vp, i, C.c_int64, C.c_int64, vp, vp, vp, vp]
     lib.gd_max_chunk.restype = i
     lib.gd_debug_divmagic.argtypes = [C.c_uint, C.c_uint, C.c_uint]
     lib.gd_debug_divmagic.restype = C.c_longlong

@@ -10,7 +10,7 @@ PKG = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CSRC = os.path.join(PKG, 'csrc')
 LIB = os.path.join(PKG, 'gdeconv', 'libgdeconv.so')
 STAMP = LIB + '.srchash'
-SOURCES = ['api.cu', 'fft_kernels.cu', 'subnet.cu', 'conv_simt.cu', 'conv_umma.cu', 'conv_l1chain.cu', 'conv_l2chain.cu', 'xdense.cu', 'synth.cu', 'shape.cu', 'fpfs.cu', 'metacal.cu']
+SOURCES = ['api.cu', 'fft_kernels.cu', 'subnet.cu', 'conv_simt.cu', 'conv_umma.cu', 'conv_l1chain.cu', 'conv_l2chain.cu', 'xdense.cu', 'synth.cu', 'shape.cu', 'fpfs.cu', 'metacal.cu', 'metacal_fixnoise.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17', '--use_fast_math=false',
               '-Xcompiler', '-fPIC', '-Xcompiler', '-fvisibility=hidden', '--expt-relaxed-constexpr']
 

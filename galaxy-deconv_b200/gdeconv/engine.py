@@ -568,16 +568,27 @@ def fpfs(img, psf=None, sigma=3.5, const=0.0):
     return dict(modes=modes, e=e, R=R, g=g)
 
 
-def metacal(img, psf=None, delta=0.01, reconv_sigma=2.5, guess_sigma=3.0, images=False):
+def metacal(img, psf=None, delta=0.01, reconv_sigma=2.5, guess_sigma=3.0, images=False, noise_sigma=None, noise=None, seed=0, start=0):
     """Metacalibration of every stamp (gd_metacal, csrc/metacal.cu): ``img`` deconvolved by ``psf`` (None: no deconvolution, for
     stamps that are already deconvolved), sheared by (0,0), (+delta,0), (-delta,0), (0,+delta), (0,-delta), reconvolved with a
     round Gaussian of sigma ``reconv_sigma`` px (one for the whole call) and measured with adaptive moments started at
     ``guess_sigma`` px.  ``img`` is fp32 CUDA [B,1,48,48], ``psf`` None, [1,1,48,48] or [B,1,48,48] on the same device (its
     normalisation does not matter; it is centred on pixel (24, 24)).  The work runs on the current stream of img's device.
+
+    Fix-noise (gd_metacal_fixnoise, Sheldon & Huff 2017): with ``noise_sigma`` or ``noise`` (not both), image j becomes
+    T_j(img) + rot90^-1(T_j(rot90(n))) for a noise field n of each stamp, which cancels the response of the sheared noise; the
+    images then carry twice the stamp's noise variance.  ``noise_sigma`` (a float, or fp32 CUDA [1] or [B]) generates
+    n = sigma N(start + i, p) from the counter hash of gdsynth on streams 60 / 61 and ``seed`` (a negative sigma negates the field, a
+    non-finite one fails the stamp); ``noise`` is the caller's unrotated field, fp32 CUDA [B,1,48,48] (for a Wiener output pass the
+    Wiener filter of sigma N).  With neither, the call is gd_metacal.
+
     Returns a dict: e [B,5,2] and status, n_iter [B,5] int32 (_lib.SHAPE_*) of the five images in that order, the response
     R [B,2,2] with R[:, i, j] = (e_i(+delta_j) - e_i(-delta_j)) / (2 delta), the per-galaxy shear g [B,2] = R^-1 e(noshear) (NaN
     unless all five statuses are OK) and, with ``images=True``, the five images [B,5,1,48,48].  The shear of an ensemble is
     mean(R)^-1 mean(e(noshear)) over the stamps whose five statuses are OK."""
+    if noise is not None and noise_sigma is not None:
+        raise ValueError('metacal: pass noise or noise_sigma, not both')
+    fix = noise is not None or noise_sigma is not None
     img = require_cuda_stamps('img', img)
     B, dev = img.shape[0], img.device
     if psf is not None:
@@ -588,11 +599,28 @@ def metacal(img, psf=None, delta=0.01, reconv_sigma=2.5, guess_sigma=3.0, images
             raise ValueError(f'psf must have batch 1 or {B}, got {psf.shape[0]}')
         if B == 0:
             psf = None
+    if noise is not None:
+        if torch.is_tensor(noise) and noise.is_cuda and noise.device != dev:
+            raise ValueError(f'noise is on {noise.device}, img on {dev}')
+        noise = require_cuda_stamps('noise', noise, B)
+    if noise_sigma is not None:
+        if torch.is_tensor(noise_sigma):
+            if not noise_sigma.is_cuda or noise_sigma.device != dev or noise_sigma.dtype != torch.float32:
+                raise ValueError(f'noise_sigma must be a float or an fp32 tensor on {dev}, got {noise_sigma.dtype} on {noise_sigma.device}')
+            if noise_sigma.dim() != 1 or noise_sigma.shape[0] not in (1, B):
+                raise ValueError(f'noise_sigma must have shape [1] or [{B}], got {tuple(noise_sigma.shape)}')
+            noise_sigma = noise_sigma.detach().contiguous()
+        else:
+            noise_sigma = torch.full((1,), float(noise_sigma), device=dev)
     ims = torch.empty(B, 5, 1, STAMP, STAMP, device=dev) if images else None
     shape = torch.empty(B, 5, 8, device=dev)
     info = torch.empty(B, 5, 2, dtype=torch.int32, device=dev)
     with torch.cuda.device(dev):
-        if B:
+        if B and fix:
+            check(lib.gd_metacal_fixnoise(_ptr(img), _ptr(psf), 0 if psf is None else psf.shape[0], B, float(delta), float(reconv_sigma),
+                                          float(guess_sigma), _ptr(noise), _ptr(noise_sigma), 0 if noise_sigma is None else noise_sigma.shape[0],
+                                          int(start), int(seed), _ptr(ims), _ptr(shape), _ptr(info), _stream(dev)))
+        elif B:
             check(lib.gd_metacal(_ptr(img), _ptr(psf), 0 if psf is None else psf.shape[0], B, float(delta), float(reconv_sigma),
                                  float(guess_sigma), _ptr(ims), _ptr(shape), _ptr(info), _stream(dev)))
         e, status = shape[:, :, 6:8], info[:, :, 0]

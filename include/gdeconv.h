@@ -205,7 +205,7 @@ GD_API int gd_fpfs(const float* img, const float* psf, int psf_batch, int batch,
  *   Re ifft2(M_j (-1)^(u+v)),   M_j(k) = I~(A_j k) G~(k) / P(A_j k),   P = p~ / p~(0)
  * with M_j = 0 where |P|^2 < 1e-8 and on the Nyquist row and column (psf NULL: P = 1).  The response is
  * R[i][j] = (e_i(+d_j) - e_i(-d_j)) / (2 d) and the shear g = R^-1 e(noshear); of an ensemble, <R>^-1 <e(noshear)> over the stamps
- * whose five statuses are GD_SHAPE_OK.  No noise-bias ("fix-noise") correction.
+ * whose five statuses are GD_SHAPE_OK.  No noise-bias correction: gd_metacal_fixnoise applies it.
  *   img    [batch][48*48] fp32 device;  psf [psf_batch][48*48] fp32 device, psf_batch 1 (one PSF for all) or batch; NULL <=> psf_batch 0
  *   delta  in (0, 0.1];  reconv_sigma, guess_sigma (the adaptive-moments start) finite, in (0, 24] px
  *   images [batch][5][48*48] fp32 device or NULL;  shape [batch][5][8] fp32 device, gd_adaptive_moments' record of each image;
@@ -213,6 +213,26 @@ GD_API int gd_fpfs(const float* img, const float* psf, int psf_batch, int batch,
  * A stamp's result does not depend on the batch it is measured in, nor on whether its PSF is given once or repeated. */
 GD_API int gd_metacal(const float* img, const float* psf, int psf_batch, int batch, float delta, float reconv_sigma, float guess_sigma,
                       float* images, float* shape, int32_t* info, void* stream);
+
+/* gd_metacal with the fix-noise correction of Sheldon & Huff 2017.  Metacalibration shears the stamp's noise with the galaxy and
+ * adaptive moments respond to sheared noise as to a shear, which biases R and g.  With rot(a)[r][c] = a[c][47 - r] (numpy's rot90),
+ * T_j the map of gd_metacal from a stamp to its image j and n a noise field of the stamp's kind, image j is
+ *   T_j(img) + rot^-1(T_j(rot n))          (the second term with the stamp's own PSF)
+ * A quarter turn flips the sign of a shear, so the two noise terms are sheared in opposite senses and their responses cancel.
+ * The shapes, R and g are gd_metacal's, on these five images; the images carry twice the noise variance of the stamp.
+ * Exactly one noise source is given:
+ *   noise        [batch][48*48] fp32 device, unrotated: the caller's field of each stamp.  Use it for stamps whose noise is not
+ *                white: for a Wiener output W(y) (linear in y at fixed alpha) pass W(sigma N) with the stamp's PSF and alpha.
+ *   noise_sigma  [sigma_batch] fp32 device, sigma_batch 1 (one sigma for all) or batch: the field of stamp i is generated,
+ *                n_i[p] = sigma_i N(start + i, p), N the standard normal of gdsynth._hashed_normal with key idx * 4099 + p on
+ *                streams 60 / 61 and `seed` (gd_synth_batch's obs noise uses streams 40 / 41, so the two are independent under any
+ *                seed).  A negative sigma negates the field; a non-finite sigma makes the stamp's images NaN (status
+ *                GD_SHAPE_FLUX on all five).  A stamp's field depends only on (seed, start + i).
+ * sigma_batch is 0 with `noise`; start >= 0 and start + batch <= INT64_MAX.  The other arguments are gd_metacal's.
+ * A stamp's result does not depend on the batch it is measured in, nor on whether its PSF or sigma is given once or repeated. */
+GD_API int gd_metacal_fixnoise(const float* img, const float* psf, int psf_batch, int batch, float delta, float reconv_sigma,
+                               float guess_sigma, const float* noise, const float* noise_sigma, int sigma_batch, int64_t start,
+                               int64_t seed, float* images, float* shape, int32_t* info, void* stream);
 
 /* Test hook: one tap-GEMM layer of the denoiser on caller-packed operands (layouts of csrc/gd_common.cuh:
  * activations [Kt/CH][Ptot][CH], CH = 8 halves (fp16 modes) or 4 floats; weights as gd_pack_weights lays them out
