@@ -1,7 +1,10 @@
 """Every tuning switch of the tcgen05 conv kernel stays a valid implementation: the product configuration and each
 alternative (cluster multicast of 1 or 2 CTAs instead of 4, epilogue prefetch placement) reproduce the golden
 UnrolledADMMGaussian(4) output of the real reference within the BASELINE tolerance, and so do both classical-solver
-kernels.  The switches are read once per process, so each variant runs in a subprocess."""
+kernels.  The switches move weights (cluster size, prefetch placement, ring depth), not sums, so each variant's ResUNet
+output is bit-identical to the default's on both layer graphs.  The switches are read once per process, so each variant
+runs in a subprocess."""
+import functools
 import json
 import os
 import subprocess
@@ -39,7 +42,16 @@ ref = O.UnrolledADMMGaussian(4).eval(); ref.load_state_dict(sd)
 with torch.no_grad():
     want = ref(b['obs'][idx].cpu(), b['psf'][idx].cpu(), b['alpha'][idx].cpu())
 err_big = float(rel_l2(big[idx].cpu(), want).max())
-print(json.dumps({'golden': err_golden, 'big': err_big, 'finite': bool(torch.isfinite(big).all())}))
+# one fixed ResUNet output per layer graph (chain: nc 32..256, fused: nc 64..512), hashed bit for bit
+import hashlib
+from models.ResUNet import ResUNet
+hashes = {}
+for name, nc in (('chain', [32, 64, 128, 256]), ('fused', [64, 128, 256, 512])):
+    r = ResUNet(nc=nc).eval()
+    r.load_state_dict(O.seeded_state_dict(lambda: O.ResUNet(nc=nc), 29))
+    z = r.to(dev)(b['obs']).cpu().contiguous()
+    hashes[name] = hashlib.sha256(z.numpy().tobytes()).hexdigest()
+print(json.dumps({'golden': err_golden, 'big': err_big, 'finite': bool(torch.isfinite(big).all()), 'hashes': hashes}))
 '''
 
 VARIANTS = [
@@ -48,14 +60,22 @@ VARIANTS = [
     {'GDECONV_CLUSTER': '2'},
     {'GDECONV_LATEPF': '0'},
     {'GDECONV_LATEPF': '1'},
+    {'GDECONV_BSTAGES': '3'},
 ]
+
+
+@functools.lru_cache(maxsize=None)
+def _run_child(env_items):
+    r = subprocess.run([sys.executable, '-c', CHILD, ROOT], env=dict(os.environ, **dict(env_items)), capture_output=True, text=True,
+                       timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    return json.loads(r.stdout.strip().splitlines()[-1])
 
 
 @pytest.mark.parametrize('env', VARIANTS, ids=lambda e: ','.join(f'{k[8:]}={v}' for k, v in e.items()) or 'default')
 def test_switch_variant_matches_reference(env):
-    r = subprocess.run([sys.executable, '-c', CHILD, ROOT], env=dict(os.environ, **env), capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stderr[-2000:]
-    res = json.loads(r.stdout.strip().splitlines()[-1])
+    res = _run_child(tuple(sorted(env.items())))
+    assert res['hashes'] == _run_child(())['hashes'], res      # bit-identical ResUNet outputs on both graphs
     assert res['finite']
     assert res['golden'] < 1e-3, res          # BASELINE tolerance: relative L2 per stamp
     assert res['big'] < 1e-3, res

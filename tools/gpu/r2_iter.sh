@@ -2,7 +2,7 @@
 # Round-2 iteration pass: chain-kernel debug, headline bench (A/B switches as arguments "ENV=VAL"), per-layer ncu table.
 #   gpurun --timeout 1200 -- 'bash tools/gpu/r2_iter.sh [ENV=VAL ...]'
 mkdir -p gpurun_out
-timeout 300 python tools/gpu/dbg_l1chain.py > gpurun_out/dbg1.log 2>&1; echo "dbg rc=$?"; grep -v "row bands" gpurun_out/dbg1.log | tail -4
+timeout 600 python -m pytest -q tests/test_resunet_rounding.py 2>&1 | tail -4
 timeout 300 python bench.py --steps 4 --warmup 3 --no-cpu-baseline > gpurun_out/b_default.json 2> gpurun_out/b1.err; echo "bench rc=$?"; cut -c1-180 gpurun_out/b_default.json
 for kv in "$@"; do
   timeout 300 env $kv python bench.py --steps 4 --warmup 3 --no-cpu-baseline > "gpurun_out/b_${kv}.json" 2>> gpurun_out/b1.err; echo "bench $kv rc=$?"; cut -c1-180 "gpurun_out/b_${kv}.json"
